@@ -4,6 +4,7 @@
 C = 16,32,64,128,256 at full 512x512 resolution; SURVEY.md §8d).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--scaling weak|strong] [--no-sustained] [--no-extra]
+                    [--dump-outputs DIR]
 
 A step = one pass of the hot path over one batch: AdaIN on the deepest level + `prev + AdaIN` on the
 four shallower ones (network/adain_rp.py:286-302 with the decoder convolutions factored out), five
@@ -18,6 +19,9 @@ Beside the headline the same line carries (all measured inside this run):
   train        config-#5-shaped training transform (AdaIN fwd+bwd + loss statistics) with the 3.1 MB gradient
                all-reduce overlapped with the backward pass — the only collective of the path
   strong       32 images in total split over the N ranks (strong scaling of the headline step)
+
+--dump-outputs DIR writes what rank 0's last timed step returned, one float32 file per level (DIR/out_c<C>.npy), so
+that two builds run with the same arguments can be compared output for output (see dump_outputs).
 """
 from __future__ import annotations
 
@@ -189,6 +193,25 @@ def make_step(torch, rpst, dev, batch, seed):
     return step, (cs, ss, ps, outs)
 
 
+DUMP_ELEMS = 1 << 21        # per level: 5 x 8 MiB of float32 stays under 64 MB in all
+DUMP_SEED = 7
+
+
+def dump_outputs(path, outs):
+    """Write one output per level as <path>/out_c<C>.npy (float32, flattened NCHW order).  A level with more than
+    DUMP_ELEMS elements is sampled at DUMP_ELEMS distinct element indices drawn with DUMP_SEED and sorted, so the
+    sample depends only on the output's size and files of two runs with the same arguments line up."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    for c, out in zip(LEVELS, outs):
+        flat = out.reshape(-1)
+        if flat.numel() > DUMP_ELEMS:
+            idx = np.sort(np.random.default_rng(DUMP_SEED).choice(flat.numel(), DUMP_ELEMS, replace=False))
+            flat = flat[torch.from_numpy(idx).to(flat.device)]
+        np.save(os.path.join(path, f"out_c{c}.npy"), flat.float().cpu().numpy())
+
+
 def train_leg(torch, dist, rpst, dev, world, steps=6):
     """Config-#5-shaped training transform on every rank (one 1024x2048 image, C=256 level): AdaIN forward,
     loss statistics (style + normalised content loss, network/adain_rp.py:81-88), backward through both, and the
@@ -320,6 +343,8 @@ def run_b200(args):
         per_level_ms[LEVELS[l]] += a.elapsed_time(b)
     kernel_ms = sum(per_level_ms.values())
     value = world * batch * args.steps / (elapsed_ms / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outs)        # before the legs below run the step again
 
     # ---- sustained: the same step for >= 2 s (the burst above lasts ~0.3 s; the power cap settles later)
     sustained = None
@@ -474,7 +499,12 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-sustained", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the configs / e2e_images / train / strong legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write rank 0's outputs of the last step as DIR/out_c<C>.npy "
+                         "(float32, a fixed seeded sample of at most 2^21 elements per level)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -41,6 +41,29 @@ def test_both_arms_name_the_same_workload():
     assert bench.algorithmic_bytes(32) == 57982058496       # SURVEY §8d: 54 GiB per 32-image step
 
 
+def test_dump_outputs_sample_is_fixed_and_bounded(tmp_path):
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    outs = [torch.arange(n, dtype=torch.float64) for n in (3, 4, 5, 6, bench.DUMP_ELEMS + 1000)]
+    bench.dump_outputs(str(tmp_path / "a"), outs)
+    bench.dump_outputs(str(tmp_path / "b"), outs)
+    for c, o in zip(bench.LEVELS, outs):
+        a, b = np.load(tmp_path / "a" / f"out_c{c}.npy"), np.load(tmp_path / "b" / f"out_c{c}.npy")
+        assert a.dtype == np.float32 and np.array_equal(a, b)
+        if o.numel() <= bench.DUMP_ELEMS:
+            assert np.array_equal(a, o.numpy())
+        else:       # distinct sorted element indices (arange: value == index)
+            assert a.shape == (bench.DUMP_ELEMS,) and (np.diff(a) > 0).all() and a[-1] < o.numel()
+
+
+def test_dump_outputs_rejected_for_the_reference_arm(tmp_path):
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=120, cwd=ROOT)
+    assert out.returncode == 2 and "--dump-outputs" in out.stderr
+
+
 def test_stub_rp_network_cpu_leg_runs():
     """The CPU arm of the `e2e_images` leg: stub RP encoder/decoder + the reference's AdaIN op sequence."""
     import torch

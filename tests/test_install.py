@@ -1,16 +1,17 @@
-"""Drop-in installation into the real reference tree (development container only: needs
-/root/reference; no GPU, so only the rebinding is checked — the numerics of every replacement are
-covered by the -m gpu tests)."""
+"""Drop-in installation into the real reference tree (no GPU, so only the rebinding is checked — the numerics
+of every replacement are covered by the -m gpu tests).  All but the state-dict test need the reference tree
+itself (RPST_REFERENCE_ROOT) and skip without it."""
 import sys
 
 import pytest
 
 from oracle.reference_loader import load_reference, reference_available
 
-pytestmark = [pytest.mark.reference,
-              pytest.mark.skipif(not reference_available(), reason="/root/reference not present")]
+needs_reference = pytest.mark.skipif(not reference_available(), reason="reference tree not found (RPST_REFERENCE_ROOT)")
 
 
+@pytest.mark.reference
+@needs_reference
 def test_install_rebinds_every_namespace_and_restores():
     import rpst
     net = load_reference()
@@ -47,22 +48,31 @@ def test_install_rebinds_every_namespace_and_restores():
     assert adain_rp.MultiScaleAdaINRPNet.decode is orig_decode
 
 
-def test_state_dict_names_match_reference():
+def test_state_dict_names_match_reference(golden):
+    """Key names, order and shapes of the reference's own modules as oracle/gen_golden.py recorded them
+    (SANet / Transform / AdaptiveSANet / AdaptiveTransform at 16 planes, both clamp modules; SELayer(32)'s
+    fc[0] / fc[2] weights): reference checkpoints load unchanged."""
     import torch
     import rpst
-    load_reference()
-    sanet = sys.modules["network.sanet"]
+    g = golden("sanet")
     torch.manual_seed(0)
-    for ours, theirs in [(rpst.SANet(8), sanet.SANet(8)), (rpst.Transform(8), sanet.Transform(8)),
-                         (rpst.AdaptiveSANet(8, 64, "aea"), sanet.AdaptiveSANet(8, 64, "aea")),
-                         (rpst.AdaptiveTransform(8, 64, 16, "relu"), sanet.AdaptiveTransform(8, 64, 16, "relu")),
-                         (rpst.SELayer(32), sys.modules["network.attention"].SELayer(32))]:
-        a, b = ours.state_dict(), theirs.state_dict()
-        assert list(a.keys()) == list(b.keys())
-        assert all(a[k].shape == b[k].shape for k in a)
-        ours.load_state_dict(b)   # reference checkpoints load unchanged
+    cases = [(rpst.SANet(16), "sanet."), (rpst.Transform(16), "transform.")]
+    for mode in ("aea", "relu"):
+        cases += [(rpst.AdaptiveSANet(16, 64, ada_module=mode), f"ada_{mode}."),
+                  (rpst.AdaptiveTransform(16, 64, 16, ada_module=mode), f"adatr_{mode}.")]
+    se = golden("se")
+    cases.append((rpst.SELayer(32, reduction=16), {"fc.0.weight": se["w1"], "fc.2.weight": se["w2"]}))
+    for ours, theirs in cases:
+        if isinstance(theirs, str):
+            theirs = {k[len(theirs):]: v for k, v in g.items() if k.startswith(theirs)}
+        a = ours.state_dict()
+        assert list(a.keys()) == list(theirs.keys())
+        assert all(a[k].shape == theirs[k].shape for k in a)
+        ours.load_state_dict(theirs)   # reference checkpoints load unchanged
 
 
+@pytest.mark.reference
+@needs_reference
 def test_patched_test_respects_subclass_decode():
     """CCAM / MST / SELast / LDMS* inherit MultiScaleAdaINRPNet.test() but define their own decode(): the patched
     test() must shuffle like the reference and call THEIR decode, not the fused multiscale one."""
@@ -97,6 +107,8 @@ def test_patched_test_respects_subclass_decode():
         rpst.uninstall()
 
 
+@pytest.mark.reference
+@needs_reference
 def test_label_map_loader_matches_the_reference_png_path(tmp_path):
     """`test.py` hands PNG paths to the segment transform; the reference reads and resizes them with PIL
     (network/base.py:448-449).  The rpst loader must produce the same label maps, and the validity table the
