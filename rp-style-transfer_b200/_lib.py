@@ -79,7 +79,12 @@ DEBUG_LIB_PATH = os.path.join(PKG, "librpst_debug.so")
 DEBUG_SIGNATURES = {
     "rpst_debug_adain_schedule": (c_int, [c_int64, c_int64, c_int, c_int, c_int, P, c_int64, P, P]),
     "rpst_debug_seg_schedule": (c_int, [c_int64, c_int64, c_int64, c_int64, c_int, P, c_int64, P, P]),
+    "rpst_debug_wct_covariances_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int64]),
+    "rpst_debug_wct_covariances": (c_int, [P, c_int64, c_int64, c_int64, c_int, c_double, c_int, P, P, P, P, c_size_t, P]),
+    "rpst_debug_dgemm_batched": (c_int, [P, P, P, c_int64, c_int64, P]),
     "rpst_last_error": (c_char_p, []),
+    "rpst_set_tuning": (c_int, [c_char_p, c_int64]),     # the debug library keeps its own knobs
+    "rpst_get_tuning": (c_int64, [c_char_p]),
 }
 
 

@@ -12,7 +12,7 @@ ROOT = os.path.dirname(PKG)
 CSRC = os.path.join(PKG, "csrc")
 LIB = os.path.join(PKG, "librpst.so")
 DEBUG_LIB = os.path.join(PKG, "librpst_debug.so")    # same sources + -DRPST_DEBUG_EXPORTS: white-box test hooks only
-DEBUG_SOURCES = ("adain.cu", "seg.cu")               # translation units that carry a debug export
+DEBUG_SOURCES = ("adain.cu", "nsroot.cu", "seg.cu", "wct.cu")               # translation units that carry a debug export
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -1614,7 +1614,7 @@ int adain_fwd_impl(const float* content, const float* style, const float* prev, 
 }
 }  // namespace
 
-#ifdef RPST_DEBUG_EXPORTS   // white-box test hooks: only in librpst_debug.so (tests/test_schedule_gpu.py), never in the product library
+#ifdef RPST_DEBUG_EXPORTS   // white-box test hooks: only in librpst_debug.so (loaded by tests alone), never in the product library
 // Test hook: the ticket schedule the TMA kernel would walk for this call shape.  info = {tickets, stats items
 // per plane, apply items per plane, lag, merge lead}; tickets [max_tickets,3] receives (kind, plane, chunk) with
 // kind 0 statistics, 1 apply, 2 merge.  Used by tests/test_schedule_gpu.py to check the schedule's invariants

@@ -44,6 +44,9 @@ struct PerDeviceFlag {
     }
 };
 
+// WCT covariance kernels (cov.cu / wct.cu): production choice, or one forced (tests)
+enum CovPath : int { kCovPathAuto = 0, kCovPathTma = 1, kCovPathStaged = 2, kCovPathPack = 3 };
+
 static inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 

@@ -232,6 +232,13 @@ constexpr uint32_t kCovBoxBytes = kCovBoxRows * kTileK * sizeof(float);    // 32
 constexpr int kCovTmaConvWarps = 16;
 constexpr int kCovTmaThreads = 32 * (2 + kCovTmaConvWarps);
 
+// The in-kernel finalize sums the per-CTA partial Grams with every warp of a CTA taking one slice of them and up to
+// kCovFinalizeLoads partials per slice: it covers kCovMaxParts partials, so the cooperative grid is clamped to that.
+constexpr int kCovFinalizeSlices = kCovTmaThreads / 32;
+constexpr int kCovFinalizeLoads = 9;
+constexpr int kCovMaxParts = kCovFinalizeSlices * kCovFinalizeLoads;   // 162 >= 148 SMs of a B200
+static_assert(kCovFinalizeSlices == 18 && kCovMaxParts == 162, "finalize slice layout (red[2][18][8][32]) out of date");
+
 template <int PARTS> struct CovTmaCfg {
     static constexpr int fstages = PARTS == 2 ? 3 : 4;          // fp32 boxes
     static constexpr int ostages = PARTS == 2 ? 2 : 3;          // operand stages (hi [+ lo], 256 rows)
@@ -518,12 +525,12 @@ __global__ void __launch_bounds__(kCovTmaThreads, 1) cov_tma_kernel(const __grid
                 const float* src = p.partial + (size_t)i * p.cp + j0;
                 const size_t zstride = (size_t)p.cp * p.cp;
 #pragma unroll 1
-                for (int k0 = 0; k0 < 9; k0 += 5) {                      // 5 + 4 sector loads in flight (148 partials)
+                for (int k0 = 0; k0 < kCovFinalizeLoads; k0 += 5) {      // 5 + 4 sector loads in flight (up to 162 partials)
                     float t[5][8];
 #pragma unroll
                     for (int k = 0; k < 5; ++k) {
-                        const int z = zs + 18 * (k0 + k);
-                        if (k0 + k < 9 && z < parts) {
+                        const int z = zs + kCovFinalizeSlices * (k0 + k);
+                        if (k0 + k < kCovFinalizeLoads && z < parts) {
                             asm volatile("ld.global.cg.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
                                          : "=f"(t[k][0]), "=f"(t[k][1]), "=f"(t[k][2]), "=f"(t[k][3]), "=f"(t[k][4]), "=f"(t[k][5]),
                                            "=f"(t[k][6]), "=f"(t[k][7]) : "l"(src + (size_t)z * zstride) : "memory");
@@ -539,7 +546,7 @@ __global__ void __launch_bounds__(kCovTmaThreads, 1) cov_tma_kernel(const __grid
                 }
             }
 #pragma unroll
-            for (int e = 0; e < 8; ++e) red[(((size_t)rr * 18 + zs) * 8 + e) * 32 + jg] = a[rr][e];   // [row][slice][column][group]
+            for (int e = 0; e < 8; ++e) red[(((size_t)rr * kCovFinalizeSlices + zs) * 8 + e) * 32 + jg] = a[rr][e];   // [row][slice][column][group]
         }
         __syncthreads();
         if (zs < 16) {                                                   // thread (jg, rr = zs / 8, e = zs % 8) finishes one column
@@ -549,7 +556,7 @@ __global__ void __launch_bounds__(kCovTmaThreads, 1) cov_tma_kernel(const __grid
             if (i < p.c && j < p.c && (i < 128 || jg < 16)) {
                 double g = 0.0;
 #pragma unroll
-                for (int q = 0; q < 18; ++q) g += red[(((size_t)rr * 18 + q) * 8 + e) * 32 + jg];   // fixed order
+                for (int q = 0; q < kCovFinalizeSlices; ++q) g += red[(((size_t)rr * kCovFinalizeSlices + q) * 8 + e) * 32 + jg];   // fixed order
                 const double v = (g - s_S[i] * s_S[j] / hw) / (hw - 1.0);
                 p.cov[(size_t)i * p.c + j] = v + (i == j ? p.diag_add : 0.0);
                 if (i < 128 && j >= 128) p.cov[(size_t)j * p.c + i] = v;        // block (1,0) is the mirror of block (0,1)
@@ -712,8 +719,11 @@ int cov_shifts_batched(const float* x, int64_t n, int64_t c, int64_t hw, float* 
     return RPST_OK;
 }
 
+// path: 0 picks the kernel (the one-launch TMA kernel when the device grants a cooperative launch and the plane has at
+// least 64 k-tiles, the register-staged kernel + finalize launches otherwise); kCovPathTma / kCovPathStaged force one
+// (tests).  *taken (may be null) receives the kernel that ran.
 int cov_fused(const float* x, int64_t c, int64_t hw, int passes, double diag_add, double* cov, float* mean, void* workspace,
-              cudaStream_t st, const float* shift_in, int* barrier_zeroed) {
+              cudaStream_t st, const float* shift_in, int path, int* taken) {
     const int cp = c <= 128 ? 128 : 256;
     const int g = sm_count();
     char* w = static_cast<char*>(workspace);
@@ -750,7 +760,17 @@ int cov_fused(const float* x, int64_t c, int64_t hw, int passes, double diag_add
     }
     // small planes (fewer k-tiles than ~half the SMs): the in-kernel finalize would run on a handful of CTAs (a 64-position
     // plane: ONE CTA walking 128 rows, 0.3 ms); they keep the separate, fully parallel finalize launches
-    EncodeTiledFn encode = g_wct_cov_tma && coop_ok[dev] == 1 && grid >= 64 && hw < (1ll << 31) - 64 ? encode_tiled_fn() : nullptr;
+    const bool tma_ok = coop_ok[dev] == 1 && hw < (1ll << 31) - 64;
+    EncodeTiledFn encode = nullptr;
+    if (path == kCovPathTma) {
+        encode = tma_ok ? encode_tiled_fn() : nullptr;
+        if (!encode) {
+            set_error("wct covariance: the one-launch TMA kernel is not available on this device");
+            return RPST_ERR_UNSUPPORTED;
+        }
+    } else if (path == 0 && g_wct_cov_tma && tma_ok && grid >= 64) {
+        encode = encode_tiled_fn();
+    }
     if (encode) {
         // x as a 2-D tensor [c rows, hw positions]; boxes of 128 rows x 64 positions (256-byte row pieces)
         CUtensorMap tmap;
@@ -772,7 +792,9 @@ int cov_fused(const float* x, int64_t c, int64_t hw, int passes, double diag_add
         p.shift_in = shift_in;
         p.prof = reinterpret_cast<unsigned long long*>(g_wct_cov_prof);
         cudaLaunchConfig_t cfg{};
-        cfg.gridDim = dim3((unsigned)grid);
+        // every partial Gram must be inside the finalize's reach: at most kCovMaxParts CTAs (k-tiles are dealt round-robin
+        // over whatever grid runs)
+        cfg.gridDim = dim3((unsigned)(grid < kCovMaxParts ? grid : kCovMaxParts));
         cfg.blockDim = dim3(kCovTmaThreads);
         cfg.dynamicSmemBytes = passes == 3 ? CovTmaCfg<2>::smem : CovTmaCfg<1>::smem;
         cfg.stream = st;
@@ -783,6 +805,7 @@ int cov_fused(const float* x, int64_t c, int64_t hw, int passes, double diag_add
         cfg.numAttrs = 1;
         if (passes == 3) RPST_CUDA(cudaLaunchKernelEx(&cfg, cov_tma_kernel<2>, tmap, p));
         else RPST_CUDA(cudaLaunchKernelEx(&cfg, cov_tma_kernel<1>, tmap, p));
+        if (taken) *taken = kCovPathTma;
         return RPST_OK;
     }
     cov_shift_kernel<<<(cp + 7) / 8, 256, 0, st>>>(x, (int)c, cp, hw, shift);
@@ -796,6 +819,7 @@ int cov_fused(const float* x, int64_t c, int64_t hw, int passes, double diag_add
     RPST_CUDA(cudaGetLastError());
     cov_finalize_kernel<<<dim3((unsigned)cp, 1), 256, 0, st>>>(partial, s_sum, grid, (int)c, cp, (double)hw, diag_add, cov);
     RPST_CUDA(cudaGetLastError());
+    if (taken) *taken = kCovPathStaged;
     return RPST_OK;
 }
 

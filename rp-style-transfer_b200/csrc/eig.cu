@@ -75,6 +75,23 @@ __device__ __forceinline__ int pos_of(int blk, int r, int m) {
     return 1 + v;
 }
 
+// The rotation angle is evaluated in fp32 from the squared column norms aa, bb (~lambda^2), the dot product gg and bb - aa.
+// When aa or bb lies outside [2^-60, 2^60] all four are first scaled by a common power of two that brings aa * bb to ~1.
+// Scaling by a power of two is exact in fp32 as long as nothing leaves the normal range, so the angle, the convergence
+// value and the zero test are the same at every scale of the input either way.  (Unscaled, aa * bb overflowed fp32 for
+// lambda_i lambda_j > ~1.8e19, and such pairs counted as converged without being rotated.)  False: aa or bb is not positive.
+__device__ __forceinline__ bool angle_inputs(double aa, double bb, double gg, float& aaf, float& bbf, float& ggf, float& dif) {
+    aaf = (float)aa; bbf = (float)bb; ggf = (float)gg; dif = (float)(bb - aa);   // difference in fp64: near-degenerate pairs cancel in fp32
+    if (aaf >= 0x1p-60f && aaf <= 0x1p60f && bbf >= 0x1p-60f && bbf <= 0x1p60f) return true;
+    if (!(aa > 0.0 && bb > 0.0)) return false;
+    const int ea = (int)((__double_as_longlong(aa) >> 52) & 0x7ff), eb = (int)((__double_as_longlong(bb) >> 52) & 0x7ff);
+    int e = 2046 - ((ea + eb) >> 1);                   // biased exponent of 2^-((ea + eb) / 2 - 1023)
+    e = e < 1 ? 1 : (e > 2046 ? 2046 : e);
+    const double sc = __longlong_as_double((long long)e << 52);
+    aaf = (float)(aa * sc); bbf = (float)(bb * sc); ggf = (float)(gg * sc); dif = (float)((bb - aa) * sc);
+    return true;
+}
+
 // rotate columns x, y (length 32*ROWS, in shared memory) so that they become orthogonal; returns |cos angle|
 template <int ROWS>
 __device__ __forceinline__ double rotate_pair(double* x, double* y, int lane) {
@@ -91,14 +108,15 @@ __device__ __forceinline__ double rotate_pair(double* x, double* y, int lane) {
     aa = warp_sum_f64(aa);
     bb = warp_sum_f64(bb);
     gg = warp_sum_f64(gg);
-    // The rotation ANGLE only steers convergence (Jacobi is self-correcting), so it is evaluated in fp32;
+    // The rotation ANGLE only steers convergence (Jacobi is self-correcting), so it is evaluated in fp32 (angle_inputs);
     // orthogonality of the rotation (c^2 + s^2 = 1) is what preserves the spectrum, so c, s are fp64.
-    const float aaf = (float)aa, bbf = (float)bb, ggf = (float)gg;
+    float aaf, bbf, ggf, dif;
+    if (!angle_inputs(aa, bb, gg, aaf, bbf, ggf, dif)) return 0.0;
     const float prod = aaf * bbf;
     if (!(prod > 0.f)) return 0.0;
     const float relf = fabsf(ggf) * rsqrtf(prod);
     if (relf <= 1e-15f) return (double)relf;
-    const float zeta = (float)(bb - aa) / (2.f * ggf);   // difference in fp64: near-degenerate pairs cancel in fp32
+    const float zeta = dif / (2.f * ggf);
     const float tf = copysignf(1.f, zeta) / (fabsf(zeta) + sqrtf(fmaf(zeta, zeta, 1.f)));
     const double t = (double)tf;
     const double c = rsqrt(fma(t, t, 1.0));
@@ -127,12 +145,13 @@ __device__ __forceinline__ double rotate_pair_tracked(double (&xv)[ROWS], double
         gg = fma(xv[i], yv[i], gg);
     }
     gg = warp_sum_f64(gg);
-    const float aaf = (float)aa, bbf = (float)bb, ggf = (float)gg;
+    float aaf, bbf, ggf, dif;
+    if (!angle_inputs(aa, bb, gg, aaf, bbf, ggf, dif)) return 0.0;
     const float prod = aaf * bbf;
     if (!(prod > 0.f)) return 0.0;
     const float relf = fabsf(ggf) * rsqrtf(prod);
     if (relf <= 1e-15f) return (double)relf;
-    const float zeta = (float)(bb - aa) / (2.f * ggf);
+    const float zeta = dif / (2.f * ggf);
     const float tf = copysignf(1.f, zeta) / (fabsf(zeta) + sqrtf(fmaf(zeta, zeta, 1.f)));
     const double t = (double)tf;
     const double c = rsqrt(fma(t, t, 1.0));

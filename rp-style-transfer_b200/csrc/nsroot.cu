@@ -619,6 +619,15 @@ int ns_roots(const double* a, int64_t batch, int n, double diag_add, double lmin
 
 using namespace rpst;
 
+#ifdef RPST_DEBUG_EXPORTS   // white-box test hooks: only in librpst_debug.so (loaded by tests alone), never in the product library
+// Test hook: c[b] = a[b] b[b] (n x n fp64, row-major) through dgemm_batched, the products of the Newton-Schulz iteration and
+// of the WCT transform (DMMA kernel with 64- or 128-row tiles for even n, DFMA kernel for odd n or with ns_dmma = 0).
+extern "C" int rpst_debug_dgemm_batched(const double* a, const double* b, double* c, int64_t batch, int64_t n, void* stream) {
+    RPST_CHECK_ARG(batch > 0 && n > 0 && n <= 512 && a && b && c, "debug_dgemm_batched: bad arguments");
+    return dgemm_batched(a, b, c, batch, (int)n, static_cast<cudaStream_t>(stream));
+}
+#endif  // RPST_DEBUG_EXPORTS
+
 extern "C" size_t rpst_spd_roots_workspace_bytes(int64_t batch, int64_t n) {
     if (batch <= 0 || n <= 0 || n > 512) return 256;
     return ns_roots_workspace_bytes(batch, (int)n);

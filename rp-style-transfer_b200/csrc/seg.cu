@@ -1058,7 +1058,7 @@ __global__ void seg_schedule_dump_kernel(SegTmaParams p, int32_t* out) {
 
 using namespace rpst;
 
-#ifdef RPST_DEBUG_EXPORTS   // white-box test hooks: only in librpst_debug.so (tests/test_schedule_gpu.py), never in the product library
+#ifdef RPST_DEBUG_EXPORTS   // white-box test hooks: only in librpst_debug.so (loaded by tests alone), never in the product library
 // Test hook, see rpst_debug_adain_schedule: kind 0 content statistics, 1 style statistics, 2 apply, 3 merge;
 // info = {tickets, content items, style items, apply items, lag}.
 extern "C" int rpst_debug_seg_schedule(int64_t n, int64_t c, int64_t hw_c, int64_t hw_s, int has_prev, int32_t* tickets,

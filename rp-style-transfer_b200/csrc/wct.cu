@@ -40,7 +40,7 @@ constexpr double kWctEigTol = 1e-5;
 bool cov_fused_supported(const float* x, int64_t c, int64_t hw);
 size_t cov_fused_workspace_bytes(int64_t c);
 int cov_fused(const float* x, int64_t c, int64_t hw, int passes, double diag_add, double* cov, float* mean, void* workspace,
-              cudaStream_t st, const float* shift_in, int* barrier_zeroed);
+              cudaStream_t st, const float* shift_in, int path, int* taken);
 int cov_shifts_batched(const float* x, int64_t n, int64_t c, int64_t hw, float* shifts, cudaStream_t st);
 extern int64_t g_wct_fused_cov;
 // wct_apply.cu: out = T (x - mu_c) + mu_s with the transposed bf16 operand built on the fly
@@ -93,7 +93,7 @@ __global__ void transform_finalize_kernel(const double* __restrict__ t, const fl
 
 struct WctLayout {
     size_t stats, mean_c, mean_s, cov_tiles_hi, cov_tiles_lo, partial, cov_c, cov_s, flag, ns, eig, mats[6], t32, bias,
-        t_hi, t_lo, x_hi, x_lo, fused, shifts, barriers, t_tile, total;
+        t_hi, t_lo, x_hi, x_lo, fused, shifts, t_tile, total;
     int splits;
 };
 
@@ -135,9 +135,51 @@ WctLayout wct_layout(int64_t n, int64_t c, int64_t hw_c, int64_t hw_s) {
     l.x_lo = take(packed_operand_bytes(hw_c, c));
     l.fused = take(c <= 256 ? cov_fused_workspace_bytes(c) : 0);
     l.shifts = take((size_t)2 * n * 256 * sizeof(float));
-    l.barriers = take((size_t)2 * n * 4 * sizeof(int));
     l.total = o;
     return l;
+}
+
+// Steps 1-2 for n contiguous [c, hw] tensors: channel means mean [n, c] (fp32) and centred covariances cov [n, c, c] (fp64,
+// / (hw - 1), + diag_add on the diagonal).  path kCovPathAuto: the fused kernels of cov.cu where the shape allows (cov_fused
+// picks the one-launch TMA kernel or the register-staged one), else pack + split-K GEMM + reduce; the other values force
+// one path (tests).  *taken (may be null) receives the path that ran.  `shifts` holds n * 256 floats.
+int wct_covariances(const float* x, int64_t n, int64_t c, int64_t hw, int passes, double diag_add, int path, double* cov,
+                    float* mean, float* shifts, const WctLayout& l, char* w, int* taken, cudaStream_t st) {
+    const bool fused_ok = cov_fused_supported(x, c, hw) && (c * hw) % 4 == 0;
+    if (path == kCovPathAuto && !(g_wct_fused_cov && fused_ok)) path = kCovPathPack;
+    if (path != kCovPathPack) {
+        RPST_CHECK_ARG(fused_ok, "wct covariance: the fused kernels need c <= 256, hw >= 64, hw %% 4 == 0 and 16-byte "
+                                 "aligned rows (c %lld, hw %lld)", (long long)c, (long long)hw);
+        // 1+2. means and centred covariances from ONE pass over each tensor (cov.cu); the centring shifts of all n tensors
+        // in one small launch (inside the covariance launch they cost a grid barrier each)
+        int rc = cov_shifts_batched(x, n, c, hw, shifts, st);
+        if (rc) return rc;
+        const int cp = c <= 128 ? 128 : 256;
+        for (int64_t i = 0; i < n; ++i)
+            if ((rc = cov_fused(x + i * c * hw, c, hw, passes, diag_add, cov + i * c * c, mean + i * c, w + l.fused, st,
+                                shifts + i * cp, path, taken))) return rc;
+        return RPST_OK;
+    }
+    // 1. channel means (network/wct_rp.py:85,92)
+    int rc = rpst_stats_nchw(x, n * c, hw, 0.f, mean, nullptr, w + l.stats, l.mean_c - l.stats, st);
+    if (rc) return rc;
+    // 2. covariances
+    void* ct_hi = w + l.cov_tiles_hi;
+    void* ct_lo = w + l.cov_tiles_lo;
+    float* partial = reinterpret_cast<float*>(w + l.partial);
+    const int cc = (int)(c * c);
+    const int splits = cov_splits(c, hw);
+    for (int64_t i = 0; i < n; ++i) {
+        rc = pack_operand_shift(x + i * c * hw, c, hw, hw, 1, nullptr, mean + i * c, ct_hi, passes == 3 ? ct_lo : nullptr, st);
+        if (rc) return rc;
+        rc = gemm_packed_splitk(ct_hi, ct_lo, ct_hi, ct_lo, partial, c, c, hw, c, passes, 1.f, nullptr, nullptr, splits, c * c, st);
+        if (rc) return rc;
+        cov_reduce_kernel<<<(cc + 255) / 256, 256, 0, st>>>(partial, splits, (int)c, 1.0 / ((double)hw - 1.0), diag_add,
+                                                           cov + i * c * c);
+        RPST_CUDA(cudaGetLastError());
+    }
+    if (taken) *taken = kCovPathPack;
+    return RPST_OK;
 }
 
 }  // namespace
@@ -173,52 +215,13 @@ extern "C" int rpst_wct_fuse(const float* content, const float* style, float* ou
     int rc;
     double* cov_c = reinterpret_cast<double*>(w + l.cov_c);
     double* cov_s = reinterpret_cast<double*>(w + l.cov_s);
+    // 1+2. means and covariances (network/wct_rp.py:85-94, + I on the content side); both tensors take the same path
     const bool fused = g_wct_fused_cov && cov_fused_supported(content, c, hw_c) && cov_fused_supported(style, c, hw_s) &&
                        (c * hw_c) % 4 == 0 && (c * hw_s) % 4 == 0;
-    if (fused) {
-        // 1+2. means and centred covariances from ONE pass over each tensor (cov.cu)
-        // centring shifts of all 2n tensors in two small launches (inside the covariance launch they cost a grid barrier each)
-        float* sh_c = reinterpret_cast<float*>(w + l.shifts);
-        float* sh_s = sh_c + n * 256;
-        if ((rc = cov_shifts_batched(content, n, c, hw_c, sh_c, st))) return rc;
-        if ((rc = cov_shifts_batched(style, n, c, hw_s, sh_s, st))) return rc;
-        const int cp = c <= 128 ? 128 : 256;
-        int* bars = reinterpret_cast<int*>(w + l.barriers);          // 4 ints per covariance launch, zeroed once for the batch
-        RPST_CUDA(cudaMemsetAsync(bars, 0, (size_t)2 * n * 4 * sizeof(int), st));
-        for (int64_t i = 0; i < n; ++i) {
-            if ((rc = cov_fused(content + i * c * hw_c, c, hw_c, passes, 1.0, cov_c + i * c * c, mean_c + i * c, w + l.fused, st,
-                                sh_c + i * cp, bars + 8 * i))) return rc;
-            if ((rc = cov_fused(style + i * c * hw_s, c, hw_s, passes, 0.0, cov_s + i * c * c, mean_s + i * c, w + l.fused, st,
-                                sh_s + i * cp, bars + 8 * i + 4))) return rc;
-        }
-    } else {
-    // 1. channel means (network/wct_rp.py:85,92)
-    rc = rpst_stats_nchw(content, n * c, hw_c, 0.f, mean_c, nullptr, w + l.stats, l.mean_c - l.stats, stream);
-    if (rc) return rc;
-    rc = rpst_stats_nchw(style, n * c, hw_s, 0.f, mean_s, nullptr, w + l.stats, l.mean_c - l.stats, stream);
-    if (rc) return rc;
-    // 2. covariances
-    void* ct_hi = w + l.cov_tiles_hi;
-    void* ct_lo = w + l.cov_tiles_lo;
-    float* partial = reinterpret_cast<float*>(w + l.partial);
-    const int cc = (int)(c * c);
-    for (int64_t i = 0; i < n; ++i) {
-        for (int which = 0; which < 2; ++which) {
-            const int64_t hw = which ? hw_s : hw_c;
-            const float* x = (which ? style : content) + i * c * hw;
-            const float* mu = (which ? mean_s : mean_c) + i * c;
-            rc = pack_operand_shift(x, c, hw, hw, 1, nullptr, mu, ct_hi, passes == 3 ? ct_lo : nullptr, st);
-            if (rc) return rc;
-            const int splits = cov_splits(c, hw);
-            rc = gemm_packed_splitk(ct_hi, ct_lo, ct_hi, ct_lo, partial, c, c, hw, c, passes, 1.f, nullptr, nullptr,
-                                    splits, c * c, st);
-            if (rc) return rc;
-            cov_reduce_kernel<<<(cc + 255) / 256, 256, 0, st>>>(partial, splits, (int)c, 1.0 / ((double)hw - 1.0),
-                                                               which ? 0.0 : 1.0, (which ? cov_s : cov_c) + i * c * c);
-            RPST_CUDA(cudaGetLastError());
-        }
-    }
-    }
+    const int path = fused ? kCovPathAuto : kCovPathPack;
+    float* shifts = reinterpret_cast<float*>(w + l.shifts);
+    if ((rc = wct_covariances(content, n, c, hw_c, passes, 1.0, path, cov_c, mean_c, shifts, l, w, nullptr, st))) return rc;
+    if ((rc = wct_covariances(style, n, c, hw_s, passes, 0.0, path, cov_s, mean_s, shifts + n * 256, l, w, nullptr, st))) return rc;
     // 3. transform matrices, batched over samples (all fp64)
     double* m[6];
     for (int i = 0; i < 6; ++i) m[i] = reinterpret_cast<double*>(w + l.mats[i]);
@@ -277,3 +280,33 @@ extern "C" int rpst_wct_fuse(const float* content, const float* style, float* ou
     }
     return RPST_OK;
 }
+
+#ifdef RPST_DEBUG_EXPORTS   // white-box test hooks: only in librpst_debug.so (loaded by tests alone), never in the product library
+extern "C" size_t rpst_debug_wct_covariances_workspace_bytes(int64_t n, int64_t c, int64_t hw) {
+    return rpst_wct_workspace_bytes(n, c, hw, hw);
+}
+
+// Test hook: steps 1-2 of rpst_wct_fuse (the same wct_covariances call) on one batch of n [c, hw] tensors, with the
+// covariance path chosen by `path` (0 production dispatch, 1 one-launch TMA kernel at any grid, 2 register-staged kernel +
+// finalize launches, 3 pack + split-K GEMM + reduce).  *path_taken (host) receives the path that ran.
+extern "C" int rpst_debug_wct_covariances(const float* x, int64_t n, int64_t c, int64_t hw, int passes, double diag_add,
+                                          int path, double* cov_out, float* mean_out, int32_t* path_taken, void* workspace,
+                                          size_t workspace_bytes, void* stream) {
+    RPST_CHECK_ARG(n > 0 && c > 0 && c <= 512 && hw >= 2, "debug_wct_covariances: bad sizes");
+    RPST_CHECK_ARG(x && cov_out && mean_out && path_taken && workspace, "debug_wct_covariances: null pointer");
+    RPST_CHECK_ARG(passes == 1 || passes == 3, "debug_wct_covariances: passes must be 1 or 3");
+    RPST_CHECK_ARG(path >= kCovPathAuto && path <= kCovPathPack, "debug_wct_covariances: path must be 0..3");
+    RPST_CHECK_ARG((reinterpret_cast<uintptr_t>(workspace) & 255u) == 0, "debug_wct_covariances: workspace must be 256-byte aligned");
+    const WctLayout l = wct_layout(n, c, hw, hw);
+    if (workspace_bytes < l.total) {
+        set_error("debug_wct_covariances: workspace too small (%zu < %zu bytes)", workspace_bytes, l.total);
+        return RPST_ERR_WORKSPACE;
+    }
+    char* w = static_cast<char*>(workspace);
+    int taken = -1;
+    const int rc = wct_covariances(x, n, c, hw, passes, diag_add, path, cov_out, mean_out, reinterpret_cast<float*>(w + l.shifts),
+                                   l, w, &taken, static_cast<cudaStream_t>(stream));
+    *path_taken = taken;
+    return rc;
+}
+#endif  // RPST_DEBUG_EXPORTS
