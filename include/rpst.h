@@ -42,28 +42,66 @@ extern "C" {
 
 RPST_API int rpst_version(void);
 RPST_API const char* rpst_last_error(void);
-/* Tuning knobs for experiments (name -> integer value); unknown names return RPST_ERR_INVALID.
- *   "adain_lag_bytes"  bytes of content kept L2-resident between the statistics and the apply phase
- *   "adain_hints"      0/1: L2 eviction-priority hints on the streaming loads/stores
- *   "adain_ctas_per_sm" persistent CTAs per SM for the register-staged pipelined kernel
- *   "adain_path"       0: TMA-staged kernel when planes are 16-byte aligned (default), 1: register-staged
- *   "seg_lag_bytes"    segment AdaIN: bytes of content between a plane's statistics and its apply
- *   "adain_stages"     TMA shared-memory stages = consumer warp groups per CTA (2..7, 32 KiB each)
- *   "watchdog_ms"      every in-kernel spin wait traps after this many ms instead of hanging the device (default 4000);
- *                      0 disables the watchdog (debuggers, MPS time-slicing, compute-sanitizer); applies to all devices
- *   "attn_flash"       1 (default): C = 512 attention runs as one flash-style kernel when the shape allows; 0: GEMM -> rows -> GEMM
- *   "wct_fused_cov" / "wct_fused_apply"   1 (default): fused convert+centre+SYRK covariance / fused colouring apply (C <= 256)
- *   "attn_flash_prof"  device pointer to 32 x uint64 cycle counters filled by the flash kernel's pair 0 (0 = off)
- *   "wct_cov_tma"      1 (default): covariance as ONE cooperative launch with TMA-staged fp32 boxes; 0: register-staged kernel
- *                      + separate shift / row-sum / finalize launches
- *   "wct_roots_ns"     1 (default): matrix roots by Newton-Schulz for C > 64, Jacobi for the matrices it flags; 0: Jacobi only;
- *                      2: Newton-Schulz with every matrix flagged (exercises the predicated Jacobi path)
- *   "wct_ns_flagged"   (read only) matrices handed to the Jacobi path by the Newton-Schulz acceptance test since load
- *   "pw_x_tma"         1 (default): pointwise convolution stages its fp32 input tiles by tensor-map TMA when the shape
- *                      allows (C_in % 64 == 0, 16-byte aligned rows); 0: register-staged converters
- *   "ns_dmma"          1 (default): Newton-Schulz products on fp64 tensor-core MMAs (even orders); 0: DFMA kernel
- *   "eig_wide"         Jacobi block width: -1 auto, 0 / 1 force 16- / 32-column blocks
- *   "wct_cov_prof"     device pointer to 16 x uint64 %globaltimer stamps of the covariance launch (0 = off) */
+/* Tuning knobs: process-wide integers that select kernel paths and schedule parameters, for experiments and A/B
+ * comparisons; the defaults are the production choice.  rpst_set_tuning returns RPST_ERR_INVALID and leaves the knob
+ * as it was for an unknown name or a value outside the knob's range (rpst_last_error() names the range).
+ * rpst_get_tuning returns the current value, or -1 for an unknown name; -1 is also a legitimate value of "eig_wide"
+ * (and "wct_ns_flagged" reads -1 when its counter cannot be read), so -1 alone does not tell the two apart.
+ *
+ *   name                        range         default    meaning
+ * AdaIN (rpst_adain_fwd, rpst_adain_fwd_mapped, rpst_stats_nchw, rpst_adain_bwd):
+ *   "adain_path"                0..1          0          0: TMA-staged kernel when planes are 16-byte aligned, 1: register-staged
+ *                                                        kernel; 1 also turns off the segment AdaIN TMA kernel (rpst_seg_adain_fwd)
+ *   "adain_stages"              2..7          6          TMA kernel: shared-memory stages = consumer warp groups per CTA (32 KiB each)
+ *   "adain_ctas_per_sm"         2..6          4          register-staged pipelined kernel: persistent CTAs per SM
+ *   "adain_lag_bytes"           0..INT64_MAX  33554432   content bytes kept L2-resident between a plane's statistics and its
+ *                                                        apply (32 MiB); also used by the backward pass and by the
+ *                                                        register-staged segment AdaIN kernel
+ *   "adain_big_lag_bytes"       0..INT64_MAX  134217728  the same for planes of 4 MiB and more (128 MiB)
+ *   "adain_mvn_lag_bytes"       0..INT64_MAX  46137344   the same for mean_variance_norm, i.e. style == NULL (44 MiB)
+ *   "adain_hints"               0..1          1          L2 eviction-priority hints on the streaming loads / stores (the
+ *                                                        register-staged segment AdaIN kernel too)
+ *   "adain_twin_apply"          0..1          1          TMA kernel without prev: each apply item carries two content chunks
+ *   "adain_group_merge_min_spp" 0..INT64_MAX  512        TMA kernel: planes with at least this many statistics slots are merged
+ *                                                        by a whole warp group instead of one warp
+ *   "adain_merge_lead"          0..INT64_MAX  0          TMA kernel: planes between a plane's merge and its first apply, clamped
+ *                                                        to 1..lag-1; 0: lag / 2
+ * Segment AdaIN, TMA kernel (rpst_seg_adain_fwd):
+ *   "seg_lag_bytes"             0..INT64_MAX  268435456  content bytes between a plane's statistics and its apply (256 MiB)
+ *   "seg_groups"                3..4          4          consumer warp groups (= stages) per CTA
+ *   "seg_flush"                 0..2          2          final flush of the statistics: 0 shared atomics per lane, 1 warp-aggregated
+ *                                                        atomics, 2 atomic-free staged gather (mode 0 above 32 usable labels)
+ * SANet attention (rpst_sanet_attn_fwd):
+ *   "attn_flash"                0..1          1          1: C = 512 attention runs as one flash-style kernel when the shape
+ *                                                        allows; 0: GEMM -> rows -> GEMM
+ *   "attn_flash_prof"           0..INT64_MAX  0          device pointer to 32 x uint64 cycle counters filled by the flash
+ *                                                        kernel's pair 0 (0 = off)
+ * WCT (rpst_wct_fuse) and its matrix functions (rpst_spd_roots, rpst_sym_eig_fn):
+ *   "wct_fused_cov"             0..1          1          1: covariances by the fused convert+centre+SYRK kernels when the shape
+ *                                                        allows (C <= 256); 0: pack + split-K GEMM
+ *   "wct_cov_tma"               0..1          1          1: fused covariance as ONE cooperative launch with TMA-staged fp32
+ *                                                        boxes; 0: register-staged kernel + separate shift / row-sum / finalize
+ *   "wct_cov_prof"              0..INT64_MAX  0          device pointer to 16 x uint64 %globaltimer stamps of the covariance
+ *                                                        launch (0 = off)
+ *   "wct_roots_ns"              0..2          1          1: matrix roots by Newton-Schulz for C > 64, Jacobi for the matrices it
+ *                                                        flags; 0: Jacobi only; 2: Newton-Schulz with every matrix flagged
+ *                                                        (exercises the predicated Jacobi path)
+ *   "ns_dmma"                   0..1          1          1: Newton-Schulz products on fp64 tensor-core MMAs (even orders);
+ *                                                        0: DFMA kernel
+ *   "eig_wide"                  -2..2         -1         Jacobi block width: -1 auto; 0 / 1 force 16- / 32-column blocks;
+ *                                                        -2 auto and print each launch's cluster occupancy to stderr;
+ *                                                        2 16-column blocks padded to one CTA per SM, occupancy printed too
+ *   "wct_fused_apply"           0..1          1          1: colouring by the fused pointwise-convolution kernel (C <= 512);
+ *                                                        0: pack + GEMM per sample
+ * Pointwise convolution (rpst_conv1x1, and the WCT colouring):
+ *   "pw_x_tma"                  0..1          1          1: fp32 input tiles staged by tensor-map TMA when the shape allows
+ *                                                        (C_in % 64 == 0, 16-byte aligned rows); 0: register-staged converters
+ * Safety and diagnostics:
+ *   "watchdog_ms"               any           4000       every in-kernel spin wait traps after this many ms instead of hanging
+ *                                                        the device; <= 0 disables the watchdog (debuggers, MPS time-slicing,
+ *                                                        profilers that stretch waits); applies to all devices
+ *   "wct_ns_flagged"            read only                matrices handed to the Jacobi path by the Newton-Schulz acceptance
+ *                                                        test since load (reading it synchronises the device) */
 RPST_API int rpst_set_tuning(const char* name, int64_t value);
 RPST_API int64_t rpst_get_tuning(const char* name);
 

@@ -20,26 +20,10 @@
 #include "common.cuh"
 #include "plane_io.cuh"
 #include "async.cuh"
+#include "tuning.cuh"
 
 namespace rpst {
 namespace {
-
-struct Tuning {
-    int64_t lag_bytes = 32ll << 20;
-    int64_t big_lag_bytes = 128ll << 20;  // planes >= 4 MiB
-    int64_t mvn_lag_bytes = 44ll << 20;   // style == NULL (mean_variance_norm): see plan_schedule
-    int64_t hints = 1;
-    int64_t ctas_per_sm = 4;
-    int64_t path = 0;    // 0: TMA-staged kernel when alignment allows, 1: register-staged kernel
-    int64_t stages = 6;  // TMA ring depth (32 KiB per stage)
-    int64_t seg_lag_bytes = 256ll << 20;  // segment AdaIN: content bytes between statistics and apply
-    int64_t group_merge_min_spp = 512;    // see merge_plane_coef_group
-    int64_t merge_lead = 0;               // 0: lag / 2
-    int64_t twin_apply = 1;               // TMA kernel, no prev: apply items carry two content chunks (32 KiB per stage)
-    int64_t seg_groups = 4;               // consumer groups (= stages) of the segment TMA kernel
-    int64_t seg_flush = 2;                // final flush: 0 shared atomics per lane, 1 warp-aggregated, 2 staged gather (atomic-free)
-};
-Tuning g_tuning;
 
 constexpr int kItemElems = 4096;  // one work item: 16 KiB of each tensor (256 threads x 4 float4)
 
@@ -1339,20 +1323,22 @@ int64_t plan_schedule(AdainParams& p, bool use_tma) {
     // spans more planes; 8x256x512x512: 32 MiB 4.2 TB/s, 40 MiB 5.07, 44 MiB 5.18, 48 MiB 4.99 (L2 misses set in), 56 MiB 4.75
     // (tools/mvn_sweep.py)
     const bool mvn = p.style == nullptr && !p.stats_only;
-    const int64_t lag_bytes = plane_bytes >= (4ll << 20) ? g_tuning.big_lag_bytes : mvn ? g_tuning.mvn_lag_bytes : g_tuning.lag_bytes;
+    const int64_t lag_bytes = plane_bytes >= (4ll << 20) ? g_knobs.adain_big_lag_bytes
+                              : mvn                      ? g_knobs.adain_mvn_lag_bytes
+                                                         : g_knobs.adain_lag_bytes;
     int64_t lag = (lag_bytes + plane_bytes - 1) / plane_bytes;
     if (lag < 3) lag = 3;
     p.lag = (int)(lag < p.planes ? lag : p.planes);
     p.slot_elems = use_tma ? kTmaSlotElems : kItemElems;
     p.spp = (int)((p.hw + p.slot_elems - 1) / p.slot_elems);
     {
-        int64_t lead = g_tuning.merge_lead > 0 ? g_tuning.merge_lead : p.lag / 2;
+        int64_t lead = g_knobs.adain_merge_lead > 0 ? g_knobs.adain_merge_lead : p.lag / 2;
         if (lead > p.lag - 1) lead = p.lag - 1;
         if (lead < 1) lead = 1;
         p.merge_lead = (int)lead;
     }
-    p.ipa = (use_tma && !p.stats_only && p.prev == nullptr && g_tuning.twin_apply) ? (p.ipp + 1) / 2 : p.ipp;
-    p.ips = (use_tma && p.style == nullptr && g_tuning.twin_apply) ? (p.ipp + 1) / 2 : p.ipp;
+    p.ipa = (use_tma && !p.stats_only && p.prev == nullptr && g_knobs.adain_twin_apply) ? (p.ipp + 1) / 2 : p.ipp;
+    p.ips = (use_tma && p.style == nullptr && g_knobs.adain_twin_apply) ? (p.ipp + 1) / 2 : p.ipp;
     p.div_s = make_fastdiv((uint32_t)p.ips);
     p.div_s1 = make_fastdiv((uint32_t)p.ips + 1u);
     p.div_s1a = make_fastdiv((uint32_t)p.ips + 1u + (uint32_t)p.ipa);
@@ -1370,7 +1356,7 @@ int launch_pipe(AdainParams p, void* ws, size_t ws_bytes, cudaStream_t stream) {
     }
     RPST_CHECK_ARG(aligned16(ws), "adain: workspace must be 16-byte aligned");
     char* base = static_cast<char*>(ws);
-    const bool use_tma = VEC == 4 && g_tuning.path == 0;
+    const bool use_tma = VEC == 4 && g_knobs.adain_path == 0;
     const int64_t total = plan_schedule(p, use_tma);
     RPST_CHECK_ARG(total < (1ll << 31), "adain: too many work items (%lld); split the call", (long long)total);
     p.total_items = (unsigned)total;
@@ -1380,7 +1366,7 @@ int launch_pipe(AdainParams p, void* ws, size_t ws_bytes, cudaStream_t stream) {
     RPST_CUDA(cudaMemsetAsync(base, 0xff, l.part_off + (size_t)p.planes * p.spp * sizeof(float4), stream));
     int rc;
     if (use_tma) {
-        switch ((int)g_tuning.stages) {
+        switch ((int)g_knobs.adain_stages) {
             case 2: rc = launch_tma_variant<2>(p, stream); break;
             case 3: rc = launch_tma_variant<3>(p, stream); break;
             case 4: rc = launch_tma_variant<4>(p, stream); break;
@@ -1389,7 +1375,7 @@ int launch_pipe(AdainParams p, void* ws, size_t ws_bytes, cudaStream_t stream) {
             default: rc = launch_tma_variant<6>(p, stream); break;
         }
     } else {
-        switch ((int)g_tuning.ctas_per_sm) {
+        switch ((int)g_knobs.adain_ctas_per_sm) {
             case 2: rc = launch_pipe_variant<VEC, 2>(p, stream); break;
             case 3: rc = launch_pipe_variant<VEC, 3>(p, stream); break;
             case 5: rc = launch_pipe_variant<VEC, 5>(p, stream); break;
@@ -1440,7 +1426,7 @@ int launch_bwd(BwdParams p, void* ws, size_t ws_bytes, cudaStream_t stream) {
     char* base = static_cast<char*>(ws);
     p.ipp = (int)((p.hw + CHUNK - 1) / CHUNK);
     const int64_t plane_bytes = 2 * p.hw * (int64_t)sizeof(float);  // dy and content stay resident
-    int64_t lag = (g_tuning.lag_bytes + plane_bytes - 1) / plane_bytes;
+    int64_t lag = (g_knobs.adain_lag_bytes + plane_bytes - 1) / plane_bytes;
     if (lag < 3) lag = 3;
     p.lag = (int)(lag < p.planes ? lag : p.planes);
     const int64_t total = p.planes * p.ipp * 2;
@@ -1473,8 +1459,8 @@ __global__ void schedule_dump_kernel(AdainParams p, int32_t* out) {
 
 int run_adain(AdainParams p, void* ws, size_t ws_bytes, cudaStream_t stream) {
     if (p.planes == 0 || p.hw == 0) return RPST_OK;
-    p.hints = (int)g_tuning.hints;
-    p.group_merge_min_spp = (int)g_tuning.group_merge_min_spp;
+    p.hints = (int)g_knobs.adain_hints;
+    p.group_merge_min_spp = (int)g_knobs.adain_group_merge_min_spp;
     bool vec = (p.hw % 4 == 0) && aligned16(p.content) && (!p.style || aligned16(p.style)) &&
                (!p.prev || aligned16(p.prev)) && (!p.out || (aligned16(p.out) && p.out_batch_stride % 4 == 0));
     if (vec) {
@@ -1486,54 +1472,6 @@ int run_adain(AdainParams p, void* ws, size_t ws_bytes, cudaStream_t stream) {
 }
 
 }  // namespace
-
-extern int64_t g_attn_flash_prof;   // flash.cu
-extern int64_t g_eig_wide;          // eig.cu
-extern int64_t g_wct_cov_tma;       // cov.cu
-extern int64_t g_wct_cov_prof;      // cov.cu
-extern int64_t g_pw_x_tma;          // pwconv.cu
-extern int64_t g_ns_dmma;           // nsroot.cu
-extern int64_t g_wct_roots_ns;      // nsroot.cu
-int64_t g_wct_fused_apply = 1;  // 1: WCT colouring through the fused transpose+convert+GEMM kernel (wct_apply.cu), C <= 256
-int64_t g_wct_fused_cov = 1;    // 1: WCT covariances through the fused convert+centre+SYRK kernel (cov.cu) when the shape allows
-int64_t g_attn_flash = 1;   // 1: C = 512 attention takes the single-kernel flash path when the shape allows (sanet.cu)
-
-int set_adain_tuning(const char* name, int64_t v, bool set, int64_t* out) {
-    int64_t* slot = nullptr;
-    if (!strcmp(name, "adain_lag_bytes")) slot = &g_tuning.lag_bytes;
-    else if (!strcmp(name, "adain_big_lag_bytes")) slot = &g_tuning.big_lag_bytes;
-    else if (!strcmp(name, "adain_mvn_lag_bytes")) slot = &g_tuning.mvn_lag_bytes;
-    else if (!strcmp(name, "adain_hints")) slot = &g_tuning.hints;
-    else if (!strcmp(name, "adain_ctas_per_sm")) slot = &g_tuning.ctas_per_sm;
-    else if (!strcmp(name, "adain_path")) slot = &g_tuning.path;
-    else if (!strcmp(name, "adain_stages")) slot = &g_tuning.stages;
-    else if (!strcmp(name, "seg_lag_bytes")) slot = &g_tuning.seg_lag_bytes;
-    else if (!strcmp(name, "seg_flush")) slot = &g_tuning.seg_flush;
-    else if (!strcmp(name, "seg_groups")) slot = &g_tuning.seg_groups;
-    else if (!strcmp(name, "adain_twin_apply")) slot = &g_tuning.twin_apply;
-    else if (!strcmp(name, "adain_group_merge_min_spp")) slot = &g_tuning.group_merge_min_spp;
-    else if (!strcmp(name, "adain_merge_lead")) slot = &g_tuning.merge_lead;
-    else if (!strcmp(name, "attn_flash")) slot = &g_attn_flash;
-    else if (!strcmp(name, "attn_flash_prof")) slot = &g_attn_flash_prof;
-    else if (!strcmp(name, "eig_wide")) slot = &g_eig_wide;
-    else if (!strcmp(name, "wct_cov_tma")) slot = &g_wct_cov_tma;
-    else if (!strcmp(name, "wct_cov_prof")) slot = &g_wct_cov_prof;
-    else if (!strcmp(name, "pw_x_tma")) slot = &g_pw_x_tma;
-    else if (!strcmp(name, "ns_dmma")) slot = &g_ns_dmma;
-    else if (!strcmp(name, "wct_roots_ns")) slot = &g_wct_roots_ns;
-    else if (!strcmp(name, "wct_fused_cov")) slot = &g_wct_fused_cov;
-    else if (!strcmp(name, "wct_fused_apply")) slot = &g_wct_fused_apply;
-    if (!slot) return 0;
-    if (set) *slot = v;
-    if (out) *out = *slot;
-    return 1;
-}
-
-int64_t adain_tuning_value(const char* name) {
-    int64_t v = 0;
-    set_adain_tuning(name, 0, false, &v);
-    return v;
-}
 
 }  // namespace rpst
 
@@ -1663,7 +1601,7 @@ extern "C" int rpst_adain_bwd(const float* grad_out, const float* content, const
     p.dstyle = grad_style;
     p.planes = n * c;
     p.hw = hw;
-    p.hints = (int)g_tuning.hints;
+    p.hints = (int)g_knobs.adain_hints;
     const bool vec = hw % 4 == 0 && aligned16(grad_out) && aligned16(content) && aligned16(grad_content) &&
                      (!grad_style || (aligned16(style) && aligned16(grad_style)));
     cudaStream_t st = static_cast<cudaStream_t>(stream);

@@ -17,6 +17,7 @@
 #include <cuda_bf16.h>
 
 #include "common.cuh"
+#include "tuning.cuh"
 #include "umma.cuh"
 
 namespace rpst {
@@ -675,9 +676,6 @@ size_t cov_fused_workspace_bytes(int64_t c) {
            align_up(cp * sizeof(float), 256) + align_up(cp * sizeof(double), 256) + 256;   // + the grid-barrier counter
 }
 
-int64_t g_wct_cov_prof = 0;  // device pointer to 16 x uint64 time stamps (0 = off); bring-up / tuning only
-int64_t g_wct_cov_tma = 1;   // tuning knob "wct_cov_tma": 1 = TMA-staged kernel, 0 = register-staged kernel
-
 namespace {
 // cuTensorMapEncodeTiled through the runtime's driver entry-point query: librpst.so does not link libcuda
 using EncodeTiledFn = CUresult (*)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
@@ -768,7 +766,7 @@ int cov_fused(const float* x, int64_t c, int64_t hw, int passes, double diag_add
             set_error("wct covariance: the one-launch TMA kernel is not available on this device");
             return RPST_ERR_UNSUPPORTED;
         }
-    } else if (path == 0 && g_wct_cov_tma && tma_ok && grid >= 64) {
+    } else if (path == 0 && g_knobs.wct_cov_tma && tma_ok && grid >= 64) {
         encode = encode_tiled_fn();
     }
     if (encode) {
@@ -790,7 +788,7 @@ int cov_fused(const float* x, int64_t c, int64_t hw, int passes, double diag_add
         RPST_CUDA(cudaMemsetAsync(barrier, 0, sizeof(int), st));
         p.barrier = barrier; p.cov = cov; p.mean = mean; p.diag_add = diag_add; p.s_sum = s_sum; p.shift = shift;
         p.shift_in = shift_in;
-        p.prof = reinterpret_cast<unsigned long long*>(g_wct_cov_prof);
+        p.prof = reinterpret_cast<unsigned long long*>(g_knobs.wct_cov_prof);
         cudaLaunchConfig_t cfg{};
         // every partial Gram must be inside the finalize's reach: at most kCovMaxParts CTAs (k-tiles are dealt round-robin
         // over whatever grid runs)

@@ -16,6 +16,7 @@
 // shared memory): the steps are shared-memory-bandwidth bound (2 x 2 KiB read + written per pair and step).
 // All CTAs of a cluster see the same convergence value, so the sweep loop exits uniformly.
 #include "common.cuh"
+#include "tuning.cuh"
 
 namespace rpst {
 namespace {
@@ -333,8 +334,6 @@ __global__ void __launch_bounds__(256) matfn_kernel(const double* __restrict__ w
 }  // namespace
 
 // ---- internal host API -------------------------------------------------------------------------
-int64_t g_eig_wide = -1;   // tuning knob "eig_wide": -1 auto, 0 / 1 force 16- / 32-column blocks, -2 auto + print cluster occupancy
-
 int eig_padded_order(int n) {
     int np = 32;
     while (np < n) np *= 2;   // 32, 64, 128, 256, 512: cluster sizes 1, 2, 4, 8, 16
@@ -362,8 +361,8 @@ int eig_decompose(const double* a, int64_t batch, int n, double diag_add, void* 
     // co-resident at one CTA per SM (cudaOccupancyMaxActiveClusters), a 16th shares SMs: 16 x 256^2 4.43 ms against
     // 4.77 with 32-column blocks (4 CTAs per matrix, 64 SMs); from 160 CTAs on the wide blocks win (32 x 256^2: 4.94 / 5.31)
     bool wide = eig_wide_ok(np) && batch * (np / 32) > 160;
-    if (g_eig_wide >= 0 && eig_wide_ok(np)) wide = g_eig_wide == 1;
-    const bool spread = g_eig_wide == 2;   // 16-column blocks, shared memory padded so that one CTA fits per SM
+    if (g_knobs.eig_wide >= 0 && eig_wide_ok(np)) wide = g_knobs.eig_wide == 1;
+    const bool spread = g_knobs.eig_wide == 2;   // 16-column blocks, shared memory padded so that one CTA fits per SM
     const int bc = wide ? 32 : 16, cta_cols = 2 * bc;
     p.a = a; p.diag_add = diag_add; p.n = n; p.np = np; p.ctas = np / cta_cols; p.max_sweeps = 20;
     p.tol = tol > 0.0 ? tol : kEigConverged;
@@ -394,7 +393,7 @@ int eig_decompose(const double* a, int64_t batch, int n, double diag_add, void* 
                                                cudaFuncAttributeNonPortableClusterSizeAllowed, 1));                \
             configured = true;                                                                                     \
         }                                                                                                          \
-        if (g_eig_wide == -2 || g_eig_wide == 2) {                                                                                    \
+        if (g_knobs.eig_wide == -2 || g_knobs.eig_wide == 2) {                                                     \
             int nc = 0;                                                                                            \
             RPST_CUDA(cudaOccupancyMaxActiveClusters(&nc, jacobi_cluster_kernel<R, BC>, &cfg));                    \
             fprintf(stderr, "[rpst] jacobi<%d,%d>: cluster %d, max active clusters %d\n", R, BC, p.ctas, nc);      \

@@ -26,6 +26,7 @@
 #include <cuda_fp16.h>
 
 #include "common.cuh"
+#include "tuning.cuh"
 #include "umma.cuh"
 
 namespace rpst {
@@ -480,8 +481,6 @@ FlashLayout flash_layout(int64_t lc, int64_t ls, int64_t max_samples) {
 
 }  // namespace
 
-int64_t g_attn_flash_prof = 0;   // device pointer to 32 x uint64 cycle counters (0 = off); bring-up / tuning only
-
 bool flash_attn_supported(int64_t c, int64_t lc, int64_t ls) {
     return c == kFlD && lc > 0 && ls > 0 && lc % 128 == 0 && ls % kFlKeys == 0;
 }
@@ -567,7 +566,7 @@ int flash_attn_run(const float* f, const float* g, const float* h, const FlashPr
         p.lc = (int)lc; p.ls = (int)ls;
         p.qtiles = (int)(lc / 128); p.ktiles = (int)(ls / kFlKeys);
         p.items = kb * p.qtiles;
-        p.prof = reinterpret_cast<unsigned long long*>(g_attn_flash_prof);
+        p.prof = reinterpret_cast<unsigned long long*>(g_knobs.attn_flash_prof);
         int pairs = sm_count() / 2;
         if (pairs > p.items) pairs = p.items;
         if (x3) flash_attn_kernel<true><<<2 * pairs, kFlThreads, FlashCfg<true>::smem, st>>>(p);

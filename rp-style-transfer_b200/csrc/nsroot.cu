@@ -19,10 +19,9 @@
 // smallest eigenvalue far below the bound, count above the cap) is FLAGGED and the caller runs the Jacobi path for the
 // flagged matrices only (eig.cu kernels take the flag array), so the reference's |s|-and-cut semantics still hold there.
 #include "common.cuh"
+#include "tuning.cuh"
 
 namespace rpst {
-
-int64_t g_ns_dmma = 1;   // tuning knob "ns_dmma": 1 = fp64 tensor-core products (mma.sync f64) for even orders, 0 = DFMA kernel
 
 namespace {
 
@@ -482,7 +481,7 @@ __global__ void __launch_bounds__(kGThreads, 2) ns_gemm_dmma_kernel(GemmArgs g) 
 
 // rows per CTA tile of the tensor-core GEMM: 64 when the 128-row tiling would leave a third of the SMs without a CTA
 int gemm_tile_rows(int n, int batch) {
-    if ((n & 1) || !g_ns_dmma) return kGM;
+    if ((n & 1) || !g_knobs.ns_dmma) return kGM;
     const int64_t ctas = (int64_t)((n + kGM - 1) / kGM) * ((n + kGN - 1) / kGN) * batch;
     return ctas < 2 * sm_count() / 3 ? 64 : kGM;
 }
@@ -490,7 +489,7 @@ int gemm_tile_rows(int n, int batch) {
 int launch_gemm(GemmArgs g, cudaStream_t st) {
     dim3 grid((unsigned)((g.n + kGN - 1) / kGN), (unsigned)((g.n + kGM - 1) / kGM), (unsigned)(g.jobs * g.batch));
     const bool even = (g.n & 1) == 0;
-    if (even && g_ns_dmma) {
+    if (even && g_knobs.ns_dmma) {
         static PerDeviceFlag configured_on;
         bool& configured = configured_on.get();
         if (!configured) {
@@ -543,9 +542,6 @@ int launch_gemm(GemmArgs g, cudaStream_t st) {
 }
 
 }  // namespace
-
-int64_t g_wct_roots_ns = 1;   // tuning knob "wct_roots_ns": 1 Newton-Schulz roots with Jacobi for flagged matrices,
-                              // 0 Jacobi only, 2 Newton-Schulz but every matrix flagged (exercises the predicated path)
 
 int64_t ns_flagged_total() {
     unsigned long long v = 0;
@@ -610,7 +606,7 @@ int ns_roots(const double* a, int64_t batch, int n, double diag_add, double lmin
     if ((rc = launch_gemm(g, st))) return rc;
     const int tiles_used = ((n + gemm_tile_rows(n, (int)batch) - 1) / gemm_tile_rows(n, (int)batch)) * ((n + kGN - 1) / kGN);
     ns_finish_kernel<<<dim3(eb, (unsigned)batch), 256, 0, st>>>(y[0], y[1], z[0], z[1], n, scale, nit, capped, partial, tiles_used,
-                                                                1e-14, g_wct_roots_ns == 2, root, iroot, flag);
+                                                                1e-14, g_knobs.wct_roots_ns == 2, root, iroot, flag);
     RPST_CUDA(cudaGetLastError());
     return RPST_OK;
 }

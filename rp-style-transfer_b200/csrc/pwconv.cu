@@ -24,6 +24,7 @@
 #include <cuda_bf16.h>
 
 #include "common.cuh"
+#include "tuning.cuh"
 #include "umma.cuh"
 
 namespace rpst {
@@ -528,8 +529,6 @@ __global__ void __launch_bounds__(128) pw_stats_finalize_kernel(const float* __r
 
 }  // namespace
 
-int64_t g_pw_x_tma = 1;   // tuning knob "pw_x_tma": 1 = x tiles by tensor-map TMA when the shape allows, 0 = register-staged converters
-
 bool pw_conv_supported(int64_t cin, int64_t cout) { return cin >= 1 && cin <= kPwMaxC && cout >= 1 && cout <= kPwMaxC; }
 
 struct PwArgs {
@@ -571,7 +570,7 @@ int pw_conv(const PwArgs& a, cudaStream_t st) {
     if (grid > items) grid = (int)items;
     CUtensorMap xmap;
     memset(&xmap, 0, sizeof(xmap));
-    const bool xtma = g_pw_x_tma && vec && epi != 2 && a.cin % 64 == 0 && a.hw < (1ll << 31) - 128 &&
+    const bool xtma = g_knobs.pw_x_tma && vec && epi != 2 && a.cin % 64 == 0 && a.hw < (1ll << 31) - 128 &&
                       a.b * a.cin < (1ll << 31) && tmap_encode_2d_f32(&xmap, a.x, (uint64_t)a.hw, (uint64_t)(a.b * a.cin), 128, 64);
     static PerDeviceFlag configured_on[24];
 #define RPST_PW_CASE(PARTS, VEC, EPI, XT)                                                                                 \

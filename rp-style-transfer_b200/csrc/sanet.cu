@@ -10,6 +10,7 @@
 //   'relu': P' = softmax_j(relu(P - clamp_i)),    clamp_i = (tanh(mlp_i) + 1) / 2
 // Softmax is over the STYLE axis without temperature (network/sanet.py:79,90-91).
 #include "common.cuh"
+#include "tuning.cuh"
 #include "umma.cuh"
 
 namespace rpst {
@@ -35,7 +36,6 @@ bool flash_attn_supported(int64_t c, int64_t lc, int64_t ls);
 size_t flash_attn_workspace_bytes(int64_t lc, int64_t ls, int64_t samples);
 int flash_attn_fwd(const float* f, const float* g, const float* h, float* out, int64_t b, int64_t lc, int64_t ls,
                    int passes, void* workspace, size_t workspace_bytes, cudaStream_t st);
-extern int64_t g_attn_flash;
 
 namespace {
 
@@ -557,7 +557,7 @@ extern "C" int rpst_sanet_attn_fwd(const float* f, const float* g, const float* 
     char* w = static_cast<char*>(workspace);
     // C = 512 without a materialised attention map: one flash-style kernel (the per-sample workspace of the
     // three-kernel path below always covers what it needs: packed Q, K, V only)
-    if (!attn_out && g_attn_flash && flash_attn_supported(c, lc, ls) && flash_attn_workspace_bytes(lc, ls, 1) <= workspace_bytes)
+    if (!attn_out && g_knobs.attn_flash && flash_attn_supported(c, lc, ls) && flash_attn_workspace_bytes(lc, ls, 1) <= workspace_bytes)
         return flash_attn_fwd(f, g, h, out, b, lc, ls, passes, workspace, workspace_bytes, st);
     const int64_t kb_max = group_size(b, workspace_bytes, per_sample);
     for (int64_t i = 0; i < b; i += kb_max) {

@@ -15,6 +15,7 @@
 // cnt_c/cnt_s<100, cnt_s/cnt_c<100) uses exact integer comparisons; pixels of unusable labels are
 // copied through bit-exactly.
 #include "common.cuh"
+#include "tuning.cuh"
 #include "plane_io.cuh"
 #include "async.cuh"
 
@@ -370,7 +371,8 @@ struct SegTmaParams {
     float2* slots;               // [planes][2][imax][kMaxDense] (S1, S2) per item; 0xFF-filled = not written
     int imax;                    // max(ic, is)
     float4* coef;                // [planes][256] (mu_c, a, mu_s, usable)
-    int flush_mode;              // 0: per-lane shared atomics, 1: warp-aggregated
+    int flush_mode;              // 0: per-lane shared atomics, 1: warp-aggregated, 2: staged gather (atomic-free; mode 0
+                                 // above 32 usable labels)
 };
 
 struct __align__(16) SegDesc {
@@ -1021,9 +1023,6 @@ int launch_seg_tma(const SegTmaParams& p, cudaStream_t st) {
 }
 
 }  // namespace
-
-int64_t adain_tuning_value(const char* name);
-
 }  // namespace rpst
 
 namespace rpst {
@@ -1037,7 +1036,7 @@ int64_t seg_plan_schedule(SegTmaParams& q, bool has_prev) {
     q.apply_elems = has_prev ? kSegPrevElems : kSegItemElems;
     q.ia = (int)((q.hw_c + q.apply_elems - 1) / q.apply_elems);
     const int64_t plane_bytes = q.hw_c * (int64_t)sizeof(float);
-    int64_t lag = (adain_tuning_value("seg_lag_bytes") + plane_bytes - 1) / plane_bytes;
+    int64_t lag = (g_knobs.seg_lag_bytes + plane_bytes - 1) / plane_bytes;
     if (lag < 3) lag = 3;
     q.lag = (int)(lag < planes ? lag : planes);
     return planes * ((int64_t)q.ic + q.is + 1 + q.ia);
@@ -1106,7 +1105,7 @@ extern "C" int rpst_seg_adain_fwd(const float* content, const float* style, cons
     const int64_t hw_max0 = hw_c > hw_s ? hw_c : hw_s;
     int hist_blocks0 = (int)((hw_max0 + 16383) / 16384);
     if (hist_blocks0 > 256) hist_blocks0 = 256;
-    const bool tma_ok = adain_tuning_value("adain_path") == 0 && hw_c % 16 == 0 && hw_s % 16 == 0 &&
+    const bool tma_ok = g_knobs.adain_path == 0 && hw_c % 16 == 0 && hw_s % 16 == 0 &&
                         aligned(content, 16) && aligned(style, 16) && aligned(out, 16) && (!prev || aligned(prev, 16)) &&
                         aligned(c_labels, 16) && aligned(s_labels, 16);
     const int* run_flag = nullptr;
@@ -1144,12 +1143,11 @@ extern "C" int rpst_seg_adain_fwd(const float* content, const float* style, cons
         const int64_t planes = n * c;
         seg_shift_kernel<<<(unsigned)((planes * 2 * kLabels + 255) / 256), 256, 0, st>>>(q);
         RPST_CUDA(cudaGetLastError());
-        q.flush_mode = (int)adain_tuning_value("seg_flush");
+        q.flush_mode = (int)g_knobs.seg_flush;
         const int64_t total = seg_plan_schedule(q, prev != nullptr);
         RPST_CHECK_ARG(total < (1ll << 31), "seg_adain: too many work items (%lld); split the call", (long long)total);
         q.total_items = (unsigned)total;
-        const int64_t groups = adain_tuning_value("seg_groups");
-        const int rc = groups == 3 ? launch_seg_tma<3>(q, st) : launch_seg_tma<4>(q, st);   // 4 groups x 2 stages x 20 KiB
+        const int rc = g_knobs.seg_groups == 3 ? launch_seg_tma<3>(q, st) : launch_seg_tma<4>(q, st);   // 4 groups x 2 stages x 20 KiB
         if (rc) return rc;
         // a sample with more than kMaxDense usable labels makes the slot kernel exit at once and the
         // register-staged kernel below run instead (device-side decision: no host synchronisation)
@@ -1160,7 +1158,7 @@ extern "C" int rpst_seg_adain_fwd(const float* content, const float* style, cons
     SegParams p{};
     p.content = content; p.style = style; p.c_lab = c_labels; p.s_lab = s_labels; p.prev = prev; p.out = out;
     p.n = n; p.channels = c; p.hw_c = hw_c; p.hw_s = hw_s; p.eps = eps;
-    p.hints = (int)adain_tuning_value("adain_hints");
+    p.hints = (int)g_knobs.adain_hints;
     p.ticket = reinterpret_cast<unsigned*>(base);
     p.done = reinterpret_cast<int*>(base + l.done_off);
     p.ready = p.done + n * c;
@@ -1189,7 +1187,7 @@ extern "C" int rpst_seg_adain_fwd(const float* content, const float* style, cons
     p.ipp_c = (int)((hw_c + chunk - 1) / chunk);
     p.ipp_s = (int)((hw_s + chunk - 1) / chunk);
     const int64_t plane_bytes = hw_c * (int64_t)sizeof(float);
-    int64_t lag = (adain_tuning_value("adain_lag_bytes") + plane_bytes - 1) / plane_bytes;
+    int64_t lag = (g_knobs.adain_lag_bytes + plane_bytes - 1) / plane_bytes;
     if (lag < 3) lag = 3;
     const int64_t planes = n * c;
     p.lag = (int)(lag < planes ? lag : planes);

@@ -12,6 +12,7 @@
 //      original (Li et al.) T = S^(1/2) C^(-1/2), small fp64 products on CUDA cores
 //   4. per sample: out = T.X + (mu_s - T.mu_c) as one tensor-core GEMM with a bias epilogue
 #include "common.cuh"
+#include "tuning.cuh"
 
 namespace rpst {
 
@@ -32,7 +33,6 @@ size_t ns_roots_workspace_bytes(int64_t batch, int n);
 int ns_roots(const double* a, int64_t batch, int n, double diag_add, double lmin, double* root, double* iroot, int* flag,
              void* workspace, size_t workspace_bytes, cudaStream_t st);
 int dgemm_batched(const double* a, const double* b, double* c, int64_t batch, int n, cudaStream_t st);
-extern int64_t g_wct_roots_ns;
 // Jacobi stop for the WCT's own decompositions: a sweep that saw |cos| < 1e-5 leaves ~1e-10 (quadratic convergence),
 // far below the fp32-grade covariances that go in; the public rpst_sym_eig_fn keeps 1e-8 (-> 1e-16).  One sweep less.
 constexpr double kWctEigTol = 1e-5;
@@ -42,15 +42,13 @@ size_t cov_fused_workspace_bytes(int64_t c);
 int cov_fused(const float* x, int64_t c, int64_t hw, int passes, double diag_add, double* cov, float* mean, void* workspace,
               cudaStream_t st, const float* shift_in, int path, int* taken);
 int cov_shifts_batched(const float* x, int64_t n, int64_t c, int64_t hw, float* shifts, cudaStream_t st);
-extern int64_t g_wct_fused_cov;
-// wct_apply.cu: out = T (x - mu_c) + mu_s with the transposed bf16 operand built on the fly
+// gemm.cu / pwconv.cu: out = T (x - mu_c) + mu_s with the transposed bf16 operand built on the fly
 int pack_operand_batched(const float* x, int64_t rows, int64_t k, int64_t stride_r, int64_t stride_k,
                          const float* row_scale, const float* row_shift, void* hi, void* lo, int batch, int64_t x_batch,
                          int64_t tile_batch_bytes, int64_t vec_batch, cudaStream_t stream);
 bool wct_apply_fused_supported(int64_t c, int64_t hw);
 int wct_apply_fused(const float* x, const float* mu_c, const float* mu_s, const void* t_hi, const void* t_lo, float* out,
                     int64_t n, int64_t t_batch_bytes, int64_t c, int64_t hw, int passes, cudaStream_t st);
-extern int64_t g_wct_fused_apply;
 
 namespace {
 
@@ -146,7 +144,7 @@ WctLayout wct_layout(int64_t n, int64_t c, int64_t hw_c, int64_t hw_s) {
 int wct_covariances(const float* x, int64_t n, int64_t c, int64_t hw, int passes, double diag_add, int path, double* cov,
                     float* mean, float* shifts, const WctLayout& l, char* w, int* taken, cudaStream_t st) {
     const bool fused_ok = cov_fused_supported(x, c, hw) && (c * hw) % 4 == 0;
-    if (path == kCovPathAuto && !(g_wct_fused_cov && fused_ok)) path = kCovPathPack;
+    if (path == kCovPathAuto && !(g_knobs.wct_fused_cov && fused_ok)) path = kCovPathPack;
     if (path != kCovPathPack) {
         RPST_CHECK_ARG(fused_ok, "wct covariance: the fused kernels need c <= 256, hw >= 64, hw %% 4 == 0 and 16-byte "
                                  "aligned rows (c %lld, hw %lld)", (long long)c, (long long)hw);
@@ -216,7 +214,7 @@ extern "C" int rpst_wct_fuse(const float* content, const float* style, float* ou
     double* cov_c = reinterpret_cast<double*>(w + l.cov_c);
     double* cov_s = reinterpret_cast<double*>(w + l.cov_s);
     // 1+2. means and covariances (network/wct_rp.py:85-94, + I on the content side); both tensors take the same path
-    const bool fused = g_wct_fused_cov && cov_fused_supported(content, c, hw_c) && cov_fused_supported(style, c, hw_s) &&
+    const bool fused = g_knobs.wct_fused_cov && cov_fused_supported(content, c, hw_c) && cov_fused_supported(style, c, hw_s) &&
                        (c * hw_c) % 4 == 0 && (c * hw_s) % 4 == 0;
     const int path = fused ? kCovPathAuto : kCovPathPack;
     float* shifts = reinterpret_cast<float*>(w + l.shifts);
@@ -234,7 +232,7 @@ extern "C" int rpst_wct_fuse(const float* content, const float* style, float* ou
     int* flag = reinterpret_cast<int*>(w + l.flag);
     auto roots = [&](const double* a, double lmin, double* root, double* iroot) -> int {
         const int* only = nullptr;
-        if (g_wct_roots_ns && c > 64) {          // up to 64 channels the Jacobi solve is as fast as the iteration's launches
+        if (g_knobs.wct_roots_ns && c > 64) {          // up to 64 channels the Jacobi solve is as fast as the iteration's launches
             if (int r = ns_roots(a, n, (int)c, 1e-4, lmin, root, iroot, flag, w + l.ns, l.eig - l.ns, st)) return r;
             only = flag;
         }
@@ -268,7 +266,7 @@ extern "C" int rpst_wct_fuse(const float* content, const float* style, float* ou
     RPST_CUDA(cudaGetLastError());
     rc = pack_operand_batched(t32, c, c, c, 1, nullptr, nullptr, w + l.t_hi, w + l.t_lo, (int)n, c * c, (int64_t)l.t_tile, 0, st);
     if (rc) return rc;
-    if (g_wct_fused_apply && wct_apply_fused_supported(c, hw_c))
+    if (g_knobs.wct_fused_apply && wct_apply_fused_supported(c, hw_c))
         return wct_apply_fused(content, mean_c, mean_s, w + l.t_hi, w + l.t_lo, out, n, (int64_t)l.t_tile, c, hw_c, passes, st);
     for (int64_t i = 0; i < n; ++i) {
         rc = pack_operand_shift(content + i * c * hw_c, hw_c, c, 1, hw_c, nullptr, nullptr, w + l.x_hi,

@@ -2,9 +2,11 @@
 include/rpst.h declares, the ctypes table mirrors the header, and argument validation works without
 touching a GPU."""
 import ctypes
+import json
 import os
 import re
 import subprocess
+import sys
 
 import pytest
 
@@ -85,6 +87,77 @@ def test_version_and_tuning(lib):
     rpst.set_tuning("adain_lag_bytes", old)
     with pytest.raises(rpst.RpstError):
         rpst.set_tuning("no_such_knob", 1)
+
+
+API_SRC = os.path.join(ROOT, "rp-style-transfer_b200", "csrc", "api.cu")
+INT64_MAX = 2**63 - 1
+
+
+def header_knobs():
+    """{name: (lo, hi, default)} of every ranged knob in the doc block above rpst_set_tuning in include/rpst.h."""
+    src = open(HEADER).read()
+    block = re.search(r"/\* Tuning knobs(.*?)\*/\s*RPST_API int rpst_set_tuning", src, flags=re.S).group(1)
+    num = r"(-?\d+|INT64_MAX)"
+    bound = lambda t: INT64_MAX if t == "INT64_MAX" else int(t)  # noqa: E731
+    return {m.group(1): (bound(m.group(2)), bound(m.group(3)), int(m.group(4)))
+            for m in re.finditer(rf'^ \*\s+"(\w+)"\s+{num}\.\.{num}\s+(-?\d+)\s', block, flags=re.M)}
+
+
+def table_knobs():
+    """Knob names of api.cu's table, in order."""
+    table = re.search(r"kKnobs\[\] = \{(.*?)\n\};", open(API_SRC).read(), flags=re.S).group(1)
+    rows = re.findall(r'\{"(\w+)", &Knobs::(\w+), ', table)
+    assert all(name == field for name, field in rows), rows
+    return [name for name, _ in rows]
+
+
+def test_knob_docs_match_table():
+    documented = header_knobs()
+    table = table_knobs()
+    assert len(table) == len(set(table)) >= 23
+    assert set(documented) == set(table), set(documented) ^ set(table)
+    block = re.search(r"/\* Tuning knobs(.*?)\*/", open(HEADER).read(), flags=re.S).group(1)
+    named = set(re.findall(r'^ \*\s+"(\w+)"', block, flags=re.M))
+    assert named == set(table) | {"watchdog_ms", "wct_ns_flagged"}, named ^ (set(table) | {"watchdog_ms", "wct_ns_flagged"})
+
+
+def test_knob_defaults_in_fresh_process():
+    documented = header_knobs()
+    code = ("import json, sys; sys.path.insert(0, sys.argv[1]); import rpst; "
+            "print(json.dumps({n: rpst.get_tuning(n) for n in sys.argv[2:]}))")
+    out = subprocess.run([sys.executable, "-c", code, ROOT, *documented], capture_output=True, text=True, timeout=300)
+    assert out.returncode == 0, out.stderr
+    got = json.loads(out.stdout.strip().splitlines()[-1])
+    assert got == {name: d for name, (_, _, d) in documented.items()}
+
+
+def test_knob_ranges_are_enforced(lib):
+    """Both ends of each documented range are accepted; one step outside is rejected, names the knob, the range and
+    the value, and leaves the knob as it was."""
+    documented = header_knobs()
+    assert len(documented) >= 23
+    for name, (lo, hi, _) in documented.items():
+        key = name.encode()
+        old = lib.rpst_get_tuning(key)
+        try:
+            for v in (lo, hi):
+                assert lib.rpst_set_tuning(key, v) == 0, lib.rpst_last_error()
+                assert lib.rpst_get_tuning(key) == v, name
+            for v in (lo - 1, hi + 1):
+                if v > INT64_MAX:
+                    continue
+                assert lib.rpst_set_tuning(key, v) == -1, (name, v)
+                err = lib.rpst_last_error()
+                assert all(s.encode() in err for s in (name, f"{lo}..{hi}", str(v))), err
+                assert lib.rpst_get_tuning(key) == hi, name
+        finally:
+            assert lib.rpst_set_tuning(key, old) == 0
+        assert lib.rpst_get_tuning(key) == old, name
+
+
+def test_read_only_knob_is_rejected(lib):
+    assert lib.rpst_set_tuning(b"wct_ns_flagged", 0) == -1
+    assert b"read-only" in lib.rpst_last_error()
 
 
 def test_argument_validation_without_gpu(lib):
