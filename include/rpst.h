@@ -45,15 +45,13 @@ RPST_API const char* rpst_last_error(void);
 /* Tuning knobs: process-wide integers that select kernel paths and schedule parameters, for experiments and A/B
  * comparisons; the defaults are the production choice.  rpst_set_tuning returns RPST_ERR_INVALID and leaves the knob
  * as it was for an unknown name or a value outside the knob's range (rpst_last_error() names the range).
- * rpst_get_tuning returns the current value, or -1 for an unknown name; -1 is also a legitimate value of "eig_wide"
- * (and "wct_ns_flagged" reads -1 when its counter cannot be read), so -1 alone does not tell the two apart.
+ * rpst_get_tuning returns the current value, or -1 for an unknown name ("wct_ns_flagged" also reads -1 when its counter
+ * cannot be read).
  *
  *   name                        range         default    meaning
  * AdaIN (rpst_adain_fwd, rpst_adain_fwd_mapped, rpst_stats_nchw, rpst_adain_bwd):
  *   "adain_path"                0..1          0          0: TMA-staged kernel when planes are 16-byte aligned, 1: register-staged
  *                                                        kernel; 1 also turns off the segment AdaIN TMA kernel (rpst_seg_adain_fwd)
- *   "adain_stages"              2..7          6          TMA kernel: shared-memory stages = consumer warp groups per CTA (32 KiB each)
- *   "adain_ctas_per_sm"         2..6          4          register-staged pipelined kernel: persistent CTAs per SM
  *   "adain_lag_bytes"           0..INT64_MAX  33554432   content bytes kept L2-resident between a plane's statistics and its
  *                                                        apply (32 MiB); also used by the backward pass and by the
  *                                                        register-staged segment AdaIN kernel
@@ -68,9 +66,6 @@ RPST_API const char* rpst_last_error(void);
  *                                                        to 1..lag-1; 0: lag / 2
  * Segment AdaIN, TMA kernel (rpst_seg_adain_fwd):
  *   "seg_lag_bytes"             0..INT64_MAX  268435456  content bytes between a plane's statistics and its apply (256 MiB)
- *   "seg_groups"                3..4          4          consumer warp groups (= stages) per CTA
- *   "seg_flush"                 0..2          2          final flush of the statistics: 0 shared atomics per lane, 1 warp-aggregated
- *                                                        atomics, 2 atomic-free staged gather (mode 0 above 32 usable labels)
  * SANet attention (rpst_sanet_attn_fwd):
  *   "attn_flash"                0..1          1          1: C = 512 attention runs as one flash-style kernel when the shape
  *                                                        allows; 0: GEMM -> rows -> GEMM
@@ -88,9 +83,6 @@ RPST_API const char* rpst_last_error(void);
  *                                                        (exercises the predicated Jacobi path)
  *   "ns_dmma"                   0..1          1          1: Newton-Schulz products on fp64 tensor-core MMAs (even orders);
  *                                                        0: DFMA kernel
- *   "eig_wide"                  -2..2         -1         Jacobi block width: -1 auto; 0 / 1 force 16- / 32-column blocks;
- *                                                        -2 auto and print each launch's cluster occupancy to stderr;
- *                                                        2 16-column blocks padded to one CTA per SM, occupancy printed too
  *   "wct_fused_apply"           0..1          1          1: colouring by the fused pointwise-convolution kernel (C <= 512);
  *                                                        0: pack + GEMM per sample
  * Pointwise convolution (rpst_conv1x1, and the WCT colouring):

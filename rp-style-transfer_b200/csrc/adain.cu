@@ -385,8 +385,10 @@ __device__ __forceinline__ float4 merge_plane_coef(const AdainParams& p, int64_t
     return cf;
 }
 
-template <int VEC, int MINB>
-__global__ void __launch_bounds__(kPipeThreads, MINB) adain_pipe_kernel(AdainParams p) {
+constexpr int kPipeCtasPerSm = 4;   // persistent CTAs per SM of the register-staged pipelined kernel
+
+template <int VEC>
+__global__ void __launch_bounds__(kPipeThreads, kPipeCtasPerSm) adain_pipe_kernel(AdainParams p) {
     constexpr int T = kPipeThreads;
     constexpr int NB = kItemElems / (T * kBatch * VEC);  // register batches per thread per tensor
     static_assert(NB >= 1, "item too small");
@@ -500,8 +502,8 @@ __global__ void __launch_bounds__(kPipeThreads, MINB) adain_pipe_kernel(AdainPar
 // One persistent CTA per SM.  Warp 0 is the PRODUCER: one thread takes tickets (two at a time, the
 // next request always in flight), decodes them and streams the item's 16 KiB chunks into a ring of
 // shared-memory stages with cp.async.bulk (TMA, 1-D: planes are contiguous), completion counted on
-// the stage's `full` mbarrier.  So the bytes in flight live in shared memory (STAGES x 32 KiB, up to
-// 224 KiB per SM), not in registers, and nobody blocks on a global load.  Each stage has its own
+// the stage's `full` mbarrier.  So the bytes in flight live in shared memory (kTmaStages x 32 KiB = 192 KiB
+// per SM), not in registers, and nobody blocks on a global load.  Each stage has its own
 // CONSUMER group of four warps: statistics items reduce the chunk(s) to (mean, M2) and publish the
 // 16-byte slot; apply items read content (L2 hit) and prev from the stage, the plane coefficients
 // from the descriptor (the producer bulk-copied the 16-byte coefficient slot along with the data)
@@ -510,6 +512,7 @@ __global__ void __launch_bounds__(kPipeThreads, MINB) adain_pipe_kernel(AdainPar
 // statistics and apply items), turns the chunk slots into the coefficient slot so that apply items
 // almost never have to wait.
 // ------------------------------------------------------------------------------------------
+constexpr int kTmaStages = 6;   // 32 KiB each; the stage sweep is profiles/r01_adain_tune_sweep.log
 constexpr int kTmaGroupWarps = 4;
 constexpr int kTmaGroupThreads = kTmaGroupWarps * 32;
 constexpr int kTmaSlotElems = kItemElems / kTmaGroupWarps;   // one warp summarises 1024 contiguous elements
@@ -693,21 +696,20 @@ __device__ __noinline__ void merge_plane_coef_group(const AdainParams& p, int64_
     named_bar_sync((uint32_t)barrier_id, kTmaGroupThreads);   // scratch is reused by the group's next merge item
 }
 
-// STAGES == number of consumer groups: group g owns stage g for the whole kernel, so the uses of a
+// One consumer group per stage: group g owns stage g for the whole kernel, so the uses of a
 // stage are consumed in order by one group and the single-bit mbarrier parity can never alias (a group
 // that ran two phases ahead of a shared stage would pass the parity wait on stale data).
 // GROUP_MERGE is a separate instantiation so that the small-plane kernel (the benchmark's) carries neither the
 // call nor its register/barrier footprint: with a run-time switch the 512x512 path lost 10 % (5.66 vs 6.3 TB/s).
-template <int STAGES, bool GROUP_MERGE>
-__global__ void __launch_bounds__(64 + STAGES * kTmaGroupThreads, 1) adain_tma_kernel(AdainParams p) {
-    constexpr int kTmaGroups = STAGES;
+template <bool GROUP_MERGE>
+__global__ void __launch_bounds__(64 + kTmaStages * kTmaGroupThreads, 1) adain_tma_kernel(AdainParams p) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     float* bufs = reinterpret_cast<float*>(smem_raw);
-    StageDesc* desc = reinterpret_cast<StageDesc*>(smem_raw + (size_t)STAGES * 2 * kItemElems * sizeof(float));
-    uint64_t* full = reinterpret_cast<uint64_t*>(desc + STAGES);
-    uint64_t* empty = full + STAGES;
-    DecodedItem* dec = reinterpret_cast<DecodedItem*>(empty + STAGES);
-    __shared__ double merge_scratch[GROUP_MERGE ? STAGES : 1][kTmaGroupWarps][5];
+    StageDesc* desc = reinterpret_cast<StageDesc*>(smem_raw + (size_t)kTmaStages * 2 * kItemElems * sizeof(float));
+    uint64_t* full = reinterpret_cast<uint64_t*>(desc + kTmaStages);
+    uint64_t* empty = full + kTmaStages;
+    DecodedItem* dec = reinterpret_cast<DecodedItem*>(empty + kTmaStages);
+    __shared__ double merge_scratch[GROUP_MERGE ? kTmaStages : 1][kTmaGroupWarps][5];
     // MERGE tickets of the single-warp merge bypass the stage ring: the producer posts the plane id into a
     // mailbox served by a dedicated merge warp (the last warp of the CTA).  Through the ring a merge queued
     // behind ~7 us of data items, twice per plane (statistics -> merge, merge -> apply), and that latency — not
@@ -719,7 +721,7 @@ __global__ void __launch_bounds__(64 + STAGES * kTmaGroupThreads, 1) adain_tma_k
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     if (threadIdx.x == 0) {
-        for (int s = 0; s < STAGES; ++s) {
+        for (int s = 0; s < kTmaStages; ++s) {
             mbar_init(&full[s], 1);
             mbar_init(&empty[s], kTmaGroupWarps);
         }
@@ -766,9 +768,9 @@ __global__ void __launch_bounds__(64 + STAGES * kTmaGroupThreads, 1) adain_tma_k
                     const int kind = dec[i].kind;
                     if (kind < 0) {
                         // out of work: one stop descriptor per consumer group (= per stage)
-                        for (int g = 0; g < kTmaGroups; ++g, ++seq) {
-                            const int stage = (int)(seq % STAGES);
-                            mbar_wait(&empty[stage], ((seq / STAGES) & 1u) ^ 1u);
+                        for (int g = 0; g < kTmaStages; ++g, ++seq) {
+                            const int stage = (int)(seq % kTmaStages);
+                            mbar_wait(&empty[stage], ((seq / kTmaStages) & 1u) ^ 1u);
                             desc[stage].kind = -1;
                             mbar_arrive(&full[stage]);
                         }
@@ -782,8 +784,8 @@ __global__ void __launch_bounds__(64 + STAGES * kTmaGroupThreads, 1) adain_tma_k
                     }
                     const int chunk = dec[i].chunk;
                     const int64_t plane = dec[i].plane;
-                    const int stage = (int)(seq % STAGES);
-                    mbar_wait(&empty[stage], ((seq / STAGES) & 1u) ^ 1u);
+                    const int stage = (int)(seq % kTmaStages);
+                    mbar_wait(&empty[stage], ((seq / kTmaStages) & 1u) ^ 1u);
                     StageDesc* d = &desc[stage];
                     // twin items carry two consecutive content chunks (apply without prev; statistics without style)
                     const bool twin = (kind == 1 && p.ipa != p.ipp) || (kind == 0 && p.ips != p.ipp);
@@ -823,7 +825,7 @@ __global__ void __launch_bounds__(64 + STAGES * kTmaGroupThreads, 1) adain_tma_k
         }
     }
 
-    if (warp == 1 + STAGES * kTmaGroupWarps) {
+    if (warp == 1 + kTmaStages * kTmaGroupWarps) {
         // ================================================================ merge warp (mailbox)
         for (unsigned mseq = 0;; ++mseq) {
             const int ms = (int)(mseq % kMailbox);
@@ -847,9 +849,9 @@ __global__ void __launch_bounds__(64 + STAGES * kTmaGroupThreads, 1) adain_tma_k
     const bool has_style = p.style != nullptr;
     const bool has_prev = p.prev != nullptr;
 
-    for (unsigned seq = group;; seq += kTmaGroups) {
-        const int stage = (int)(seq % STAGES);
-        const unsigned ph = (seq / STAGES) & 1u;
+    for (unsigned seq = group;; seq += kTmaStages) {
+        const int stage = (int)(seq % kTmaStages);
+        const unsigned ph = (seq / kTmaStages) & 1u;
         mbar_wait(&full[stage], ph);  // every lane observes the phase (async-proxy writes become visible to waiters)
         const StageDesc* d = &desc[stage];
         const int kind = d->kind;           // copy everything out of the descriptor: once the stage is
@@ -1268,45 +1270,36 @@ int launch_direct(const AdainParams& p, cudaStream_t stream) {
     return RPST_OK;
 }
 
-template <int VEC, int MINB>
+template <int VEC>
 int launch_pipe_variant(const AdainParams& p, cudaStream_t stream) {
     // every CTA must be co-resident (apply items poll slots written by other CTAs)
     static int blocks_per_sm = 0;
     if (blocks_per_sm == 0) {
         int nb = 0;
-        RPST_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, adain_pipe_kernel<VEC, MINB>, kPipeThreads, 0));
+        RPST_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, adain_pipe_kernel<VEC>, kPipeThreads, 0));
         blocks_per_sm = nb > 0 ? nb : 1;
     }
-    const int per_sm = blocks_per_sm < MINB ? blocks_per_sm : MINB;
+    const int per_sm = blocks_per_sm < kPipeCtasPerSm ? blocks_per_sm : kPipeCtasPerSm;
     int64_t grid = (int64_t)sm_count() * per_sm;
     if (grid > (int64_t)p.total_items) grid = p.total_items;
-    adain_pipe_kernel<VEC, MINB><<<(int)grid, kPipeThreads, 0, stream>>>(p);
+    adain_pipe_kernel<VEC><<<(int)grid, kPipeThreads, 0, stream>>>(p);
     RPST_CUDA(cudaGetLastError());
     return RPST_OK;
 }
 
-template <int STAGES, bool GROUP_MERGE>
-int launch_tma_variant2(const AdainParams& p, cudaStream_t stream);
-
-template <int STAGES>
+template <bool GROUP_MERGE>
 int launch_tma_variant(const AdainParams& p, cudaStream_t stream) {
-    return (!p.stats_only && p.spp >= p.group_merge_min_spp) ? launch_tma_variant2<STAGES, true>(p, stream)
-                                                             : launch_tma_variant2<STAGES, false>(p, stream);
-}
-
-template <int STAGES, bool GROUP_MERGE>
-int launch_tma_variant2(const AdainParams& p, cudaStream_t stream) {
-    constexpr size_t smem = (size_t)STAGES * 2 * kItemElems * sizeof(float) + STAGES * sizeof(StageDesc) +
-                            2 * STAGES * sizeof(uint64_t) + kTicketBatch * sizeof(DecodedItem);
+    constexpr size_t smem = (size_t)kTmaStages * 2 * kItemElems * sizeof(float) + kTmaStages * sizeof(StageDesc) +
+                            2 * kTmaStages * sizeof(uint64_t) + kTicketBatch * sizeof(DecodedItem);
     static PerDeviceFlag configured_on;
     bool& configured = configured_on.get();
     if (!configured) {
-        RPST_CUDA(cudaFuncSetAttribute(adain_tma_kernel<STAGES, GROUP_MERGE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        RPST_CUDA(cudaFuncSetAttribute(adain_tma_kernel<GROUP_MERGE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         configured = true;
     }
     int64_t grid = sm_count();
     if (grid > (int64_t)p.total_items) grid = p.total_items;
-    adain_tma_kernel<STAGES, GROUP_MERGE><<<(int)grid, 64 + STAGES * kTmaGroupThreads, smem, stream>>>(p);
+    adain_tma_kernel<GROUP_MERGE><<<(int)grid, 64 + kTmaStages * kTmaGroupThreads, smem, stream>>>(p);
     RPST_CUDA(cudaGetLastError());
     return RPST_OK;
 }
@@ -1365,24 +1358,9 @@ int launch_pipe(AdainParams p, void* ws, size_t ws_bytes, cudaStream_t stream) {
     p.part = reinterpret_cast<float4*>(base + l.part_off);
     RPST_CUDA(cudaMemsetAsync(base, 0xff, l.part_off + (size_t)p.planes * p.spp * sizeof(float4), stream));
     int rc;
-    if (use_tma) {
-        switch ((int)g_knobs.adain_stages) {
-            case 2: rc = launch_tma_variant<2>(p, stream); break;
-            case 3: rc = launch_tma_variant<3>(p, stream); break;
-            case 4: rc = launch_tma_variant<4>(p, stream); break;
-            case 5: rc = launch_tma_variant<5>(p, stream); break;
-            case 7: rc = launch_tma_variant<7>(p, stream); break;
-            default: rc = launch_tma_variant<6>(p, stream); break;
-        }
-    } else {
-        switch ((int)g_knobs.adain_ctas_per_sm) {
-            case 2: rc = launch_pipe_variant<VEC, 2>(p, stream); break;
-            case 3: rc = launch_pipe_variant<VEC, 3>(p, stream); break;
-            case 5: rc = launch_pipe_variant<VEC, 5>(p, stream); break;
-            case 6: rc = launch_pipe_variant<VEC, 6>(p, stream); break;
-            default: rc = launch_pipe_variant<VEC, 4>(p, stream); break;
-        }
-    }
+    if (!use_tma) rc = launch_pipe_variant<VEC>(p, stream);
+    else if (!p.stats_only && p.spp >= p.group_merge_min_spp) rc = launch_tma_variant<true>(p, stream);
+    else rc = launch_tma_variant<false>(p, stream);
     if (rc != RPST_OK) return rc;
     if (p.stats_only) {
         stats_finalize_kernel<<<(unsigned)((p.planes + 7) / 8), 256, 0, stream>>>(p);

@@ -46,15 +46,11 @@ static const KnobSpec kKnobs[] = {
     {"adain_big_lag_bytes", &Knobs::adain_big_lag_bytes, 0, INT64_MAX},
     {"adain_mvn_lag_bytes", &Knobs::adain_mvn_lag_bytes, 0, INT64_MAX},
     {"adain_hints", &Knobs::adain_hints, 0, 1},
-    {"adain_ctas_per_sm", &Knobs::adain_ctas_per_sm, 2, 6},
     {"adain_path", &Knobs::adain_path, 0, 1},
-    {"adain_stages", &Knobs::adain_stages, 2, 7},
     {"adain_twin_apply", &Knobs::adain_twin_apply, 0, 1},
     {"adain_group_merge_min_spp", &Knobs::adain_group_merge_min_spp, 0, INT64_MAX},
     {"adain_merge_lead", &Knobs::adain_merge_lead, 0, INT64_MAX},
     {"seg_lag_bytes", &Knobs::seg_lag_bytes, 0, INT64_MAX},
-    {"seg_groups", &Knobs::seg_groups, 3, 4},
-    {"seg_flush", &Knobs::seg_flush, 0, 2},
     {"attn_flash", &Knobs::attn_flash, 0, 1},
     {"attn_flash_prof", &Knobs::attn_flash_prof, 0, INT64_MAX},
     {"wct_fused_cov", &Knobs::wct_fused_cov, 0, 1},
@@ -63,7 +59,6 @@ static const KnobSpec kKnobs[] = {
     {"wct_cov_prof", &Knobs::wct_cov_prof, 0, INT64_MAX},
     {"wct_roots_ns", &Knobs::wct_roots_ns, 0, 2},
     {"ns_dmma", &Knobs::ns_dmma, 0, 1},
-    {"eig_wide", &Knobs::eig_wide, -2, 2},
     {"pw_x_tma", &Knobs::pw_x_tma, 0, 1},
 };
 

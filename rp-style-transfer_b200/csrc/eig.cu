@@ -16,7 +16,6 @@
 // shared memory): the steps are shared-memory-bandwidth bound (2 x 2 KiB read + written per pair and step).
 // All CTAs of a cluster see the same convergence value, so the sweep loop exits uniformly.
 #include "common.cuh"
-#include "tuning.cuh"
 
 namespace rpst {
 namespace {
@@ -360,15 +359,12 @@ int eig_decompose(const double* a, int64_t batch, int n, double diag_add, void* 
     // 16-column blocks (np/32 CTAs per matrix) until they need more than ~one CTA per SM; 15 eight-CTA clusters are
     // co-resident at one CTA per SM (cudaOccupancyMaxActiveClusters), a 16th shares SMs: 16 x 256^2 4.43 ms against
     // 4.77 with 32-column blocks (4 CTAs per matrix, 64 SMs); from 160 CTAs on the wide blocks win (32 x 256^2: 4.94 / 5.31)
-    bool wide = eig_wide_ok(np) && batch * (np / 32) > 160;
-    if (g_knobs.eig_wide >= 0 && eig_wide_ok(np)) wide = g_knobs.eig_wide == 1;
-    const bool spread = g_knobs.eig_wide == 2;   // 16-column blocks, shared memory padded so that one CTA fits per SM
+    const bool wide = eig_wide_ok(np) && batch * (np / 32) > 160;
     const int bc = wide ? 32 : 16, cta_cols = 2 * bc;
     p.a = a; p.diag_add = diag_add; p.n = n; p.np = np; p.ctas = np / cta_cols; p.max_sweeps = 20;
     p.tol = tol > 0.0 ? tol : kEigConverged;
     p.w = w; p.lam = lam; p.sweeps = sweeps; p.only = only;
-    size_t smem = (size_t)cta_cols * np * sizeof(double) + 2 * sizeof(double);
-    if (spread && smem < (120u << 10)) smem = 120u << 10;
+    const size_t smem = (size_t)cta_cols * np * sizeof(double) + 2 * sizeof(double);
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = dim3((unsigned)(batch * p.ctas));
     cfg.blockDim = dim3(32 * bc);
@@ -387,16 +383,11 @@ int eig_decompose(const double* a, int64_t batch, int n, double diag_add, void* 
         bool& configured = configured_on.get();                                                                    \
         if (!configured) {                                                                                         \
             RPST_CUDA(cudaFuncSetAttribute(jacobi_cluster_kernel<R, BC>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                           (int)(smem > (120u << 10) ? smem : (120u << 10))));                     \
+                                           (int)smem));                                                            \
             if (32 * R / (2 * BC) > 8)                                                                             \
                 RPST_CUDA(cudaFuncSetAttribute(jacobi_cluster_kernel<R, BC>,                                       \
                                                cudaFuncAttributeNonPortableClusterSizeAllowed, 1));                \
             configured = true;                                                                                     \
-        }                                                                                                          \
-        if (g_knobs.eig_wide == -2 || g_knobs.eig_wide == 2) {                                                     \
-            int nc = 0;                                                                                            \
-            RPST_CUDA(cudaOccupancyMaxActiveClusters(&nc, jacobi_cluster_kernel<R, BC>, &cfg));                    \
-            fprintf(stderr, "[rpst] jacobi<%d,%d>: cluster %d, max active clusters %d\n", R, BC, p.ctas, nc);      \
         }                                                                                                          \
         RPST_CUDA(cudaLaunchKernelEx(&cfg, jacobi_cluster_kernel<R, BC>, p));                                      \
         break;                                                                                                     \

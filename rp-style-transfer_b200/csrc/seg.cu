@@ -340,6 +340,7 @@ constexpr int kSegStageBytes = kSegDataBytes + kSegItemElems;       // data (+pr
 // in the wait for the stage's `full` barrier (fetch latency + producer turnaround) and the rest in processing,
 // strictly one after the other.
 constexpr int kSegDepth = 2;
+constexpr int kSegGroups = 4;   // consumer groups of seg_tma_kernel: 4 x kSegDepth stages of 20 KiB
 constexpr int kSegGroupWarps = 4;
 constexpr int kSegGroupThreads = kSegGroupWarps * 32;
 constexpr int kSegWarpVecs = kSegItemElems / 4 / kSegGroupWarps;   // 512 float4 per warp per full item
@@ -371,8 +372,6 @@ struct SegTmaParams {
     float2* slots;               // [planes][2][imax][kMaxDense] (S1, S2) per item; 0xFF-filled = not written
     int imax;                    // max(ic, is)
     float4* coef;                // [planes][256] (mu_c, a, mu_s, usable)
-    int flush_mode;              // 0: per-lane shared atomics, 1: warp-aggregated, 2: staged gather (atomic-free; mode 0
-                                 // above 32 usable labels)
 };
 
 struct __align__(16) SegDesc {
@@ -515,15 +514,14 @@ __device__ __forceinline__ void seg_warp_totals(float2* tab, int lane, int cur, 
     __syncwarp();
 }
 
-template <int G>
-__global__ void __launch_bounds__(32 + G * kSegGroupThreads + kSegMergeThreads, 1) seg_tma_kernel(SegTmaParams p) {
-    constexpr int S = G * kSegDepth;   // stages; group g owns stages g*kSegDepth .. +kSegDepth-1
+__global__ void __launch_bounds__(32 + kSegGroups * kSegGroupThreads + kSegMergeThreads, 1) seg_tma_kernel(SegTmaParams p) {
+    constexpr int S = kSegGroups * kSegDepth;   // stages; group g owns stages g*kSegDepth .. +kSegDepth-1
     constexpr int STAGE_BYTES = kSegStageBytes;
     constexpr int CACHE_BYTES = kSegCacheBytes;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     unsigned char* stages = smem_raw;
     unsigned char* caches = smem_raw + (size_t)S * STAGE_BYTES;
-    SegDesc* desc = reinterpret_cast<SegDesc*>(caches + (size_t)G * ((CACHE_BYTES + 127) / 128 * 128));
+    SegDesc* desc = reinterpret_cast<SegDesc*>(caches + (size_t)kSegGroups * ((CACHE_BYTES + 127) / 128 * 128));
     uint64_t* full = reinterpret_cast<uint64_t*>(desc + S);
     uint64_t* empty = full + S;
     uint64_t* mfull = empty + S;              // merge mailbox: producer -> merge warps
@@ -557,10 +555,10 @@ __global__ void __launch_bounds__(32 + G * kSegGroupThreads + kSegMergeThreads, 
             const unsigned base = __shfl_sync(0xffffffffu, next_base, 0);
             if (lane == 0) next_base = atomicAdd(p.ticket, (unsigned)kSegTicketBatch) + 1u;
             // Lane i decodes AND issues ticket base+i: the eight items of a batch go to eight different stages
-            // (consecutive sequence numbers, G*kSegDepth >= kSegTicketBatch), so their empty-waits, descriptors
-            // and TMA issues run in SIMT lock-step instead of one after the other on a single thread (which
+            // (consecutive sequence numbers, kSegGroups * kSegDepth >= kSegTicketBatch), so their empty-waits,
+            // descriptors and TMA issues run in SIMT lock-step instead of one after the other on a single thread (which
             // capped both TMA kernels at ~1.3 M items/s per SM).
-            static_assert(G * kSegDepth >= kSegTicketBatch || G * kSegDepth == 6, "a batch must not reuse a stage");
+            static_assert(kSegGroups * kSegDepth >= kSegTicketBatch, "a batch must not reuse a stage");
             int kind = 3, chunk = 0;    // lanes >= batch: treated like a merge (skipped)
             int64_t plane = 0;
             if (lane < kSegTicketBatch) {
@@ -587,44 +585,41 @@ __global__ void __launch_bounds__(32 + G * kSegGroupThreads + kSegMergeThreads, 
             }
             const bool is_item = lane < nvalid && kind != 3;
             const unsigned itemmask = __ballot_sync(0xffffffffu, is_item);
-            constexpr int kRound = G * kSegDepth < kSegTicketBatch ? G * kSegDepth : kSegTicketBatch;   // items issued together
             const int my_pos = __popc(itemmask & ((1u << lane) - 1u));
-            for (int r0 = 0; r0 < kSegTicketBatch; r0 += kRound) {
-                if (is_item && my_pos >= r0 && my_pos < r0 + kRound) {
-                    const unsigned my_seq = seq + (unsigned)my_pos;
-                    const unsigned k = my_seq / G;
-                    const int stage = (int)(my_seq % G) * kSegDepth + (int)(k % kSegDepth);
-                    mbar_wait_quiet(&empty[stage], ((k / kSegDepth) & 1u) ^ 1u);
-                    SegDesc* d = &desc[stage];
-                    d->plane = plane; d->kind = kind; d->chunk = chunk;
-                    const bool is_style = kind == 1;
-                    const int64_t hw = is_style ? p.hw_s : p.hw_c;
-                    const int item_elems = kind == 2 ? p.apply_elems : kSegItemElems;
-                    const int64_t e0 = (int64_t)chunk * item_elems;
-                    const int64_t rem = hw - e0;
-                    const int nvec = (int)((rem < item_elems ? rem : item_elems) / 4);
-                    d->nvec = nvec;
-                    const uint32_t bytes = (uint32_t)nvec * 16u;
-                    unsigned char* st = stages + (size_t)stage * STAGE_BYTES;
-                    const int64_t sample = (int)plane / (int)p.channels;
-                    const float* src = (is_style ? p.style : p.content) + plane * hw + e0;
-                    const uint8_t* lab = (is_style ? p.s_lab : p.c_lab) + sample * hw + e0;
-                    const bool has_prev = kind == 2 && p.prev != nullptr;
-                    mbar_arrive_expect_tx(&full[stage], bytes + (has_prev ? bytes : 0u) + (uint32_t)nvec * 4u);
-                    tma_load_1d(st, src, bytes, &full[stage], kind == 0 ? pol_last : pol_first);
-                    if (has_prev)
-                        tma_load_1d(st + kSegHalfElems * 4, p.prev + plane * hw + e0, bytes, &full[stage], pol_first);
-                    tma_load_1d(st + kSegDataBytes, lab, (uint32_t)nvec * 4u, &full[stage], pol_last);
-                }
-                __syncwarp();
+            if (is_item) {
+                const unsigned my_seq = seq + (unsigned)my_pos;
+                const unsigned k = my_seq / kSegGroups;
+                const int stage = (int)(my_seq % kSegGroups) * kSegDepth + (int)(k % kSegDepth);
+                mbar_wait_quiet(&empty[stage], ((k / kSegDepth) & 1u) ^ 1u);
+                SegDesc* d = &desc[stage];
+                d->plane = plane; d->kind = kind; d->chunk = chunk;
+                const bool is_style = kind == 1;
+                const int64_t hw = is_style ? p.hw_s : p.hw_c;
+                const int item_elems = kind == 2 ? p.apply_elems : kSegItemElems;
+                const int64_t e0 = (int64_t)chunk * item_elems;
+                const int64_t rem = hw - e0;
+                const int nvec = (int)((rem < item_elems ? rem : item_elems) / 4);
+                d->nvec = nvec;
+                const uint32_t bytes = (uint32_t)nvec * 16u;
+                unsigned char* st = stages + (size_t)stage * STAGE_BYTES;
+                const int64_t sample = (int)plane / (int)p.channels;
+                const float* src = (is_style ? p.style : p.content) + plane * hw + e0;
+                const uint8_t* lab = (is_style ? p.s_lab : p.c_lab) + sample * hw + e0;
+                const bool has_prev = kind == 2 && p.prev != nullptr;
+                mbar_arrive_expect_tx(&full[stage], bytes + (has_prev ? bytes : 0u) + (uint32_t)nvec * 4u);
+                tma_load_1d(st, src, bytes, &full[stage], kind == 0 ? pol_last : pol_first);
+                if (has_prev)
+                    tma_load_1d(st + kSegHalfElems * 4, p.prev + plane * hw + e0, bytes, &full[stage], pol_first);
+                tma_load_1d(st + kSegDataBytes, lab, (uint32_t)nvec * 4u, &full[stage], pol_last);
             }
+            __syncwarp();
             seq += (unsigned)__popc(itemmask);
             bool finished = false;
             if (stopmask != 0u) {
                 if (lane == 0) {
-                    for (int g = 0; g < G; ++g, ++seq) {   // one stop descriptor per consumer group
-                        const unsigned k = seq / G;
-                        const int stage = (int)(seq % G) * kSegDepth + (int)(k % kSegDepth);
+                    for (int g = 0; g < kSegGroups; ++g, ++seq) {   // one stop descriptor per consumer group
+                        const unsigned k = seq / kSegGroups;
+                        const int stage = (int)(seq % kSegGroups) * kSegDepth + (int)(k % kSegDepth);
                         mbar_wait_quiet(&empty[stage], ((k / kSegDepth) & 1u) ^ 1u);
                         desc[stage].kind = -1;
                         mbar_arrive(&full[stage]);
@@ -641,14 +636,14 @@ __global__ void __launch_bounds__(32 + G * kSegGroupThreads + kSegMergeThreads, 
         }
     }
 
-    if (warp > G * kSegGroupWarps) {
+    if (warp > kSegGroups * kSegGroupWarps) {
         // ================================================================ merge warps
         // The 64 merge threads split a plane's slot rows as (dense label, part): with d usable labels there are
         // 64/d parts per label, each summing a contiguous range of item slots (content then style, fixed
         // order, fp64, 32 loads in flight); part 0 then adds the parts in index order (deterministic) and
         // writes the label's coefficients.  19 labels => 3 parts => a plane's ~1000 slots take ~11 load rounds.
         __shared__ double s_merge[kSegMergeThreads][4];
-        const int t = threadIdx.x - (32 + G * kSegGroupThreads);
+        const int t = threadIdx.x - (32 + kSegGroups * kSegGroupThreads);
         for (unsigned mseq = 0;; ++mseq) {
             const int ms = (int)(mseq % kSegMailbox);
             mbar_wait_quiet(&mfull[ms], (mseq / kSegMailbox) & 1u, 64);
@@ -744,8 +739,8 @@ __global__ void __launch_bounds__(32 + G * kSegGroupThreads + kSegMergeThreads, 
     for (int i = gt; i < 2 * kMaxDense * 2; i += kSegGroupThreads) c_acc[i] = 0.f;
     named_bar_sync(1 + group, kSegGroupThreads);
 
-    for (unsigned seq = group;; seq += G) {
-        const unsigned k = seq / G;
+    for (unsigned seq = group;; seq += kSegGroups) {
+        const unsigned k = seq / kSegGroups;
         const int stage = group * kSegDepth + (int)(k % kSegDepth);
         mbar_wait_quiet(&full[stage], (k / kSegDepth) & 1u);
         const SegDesc* d = &desc[stage];
@@ -836,36 +831,17 @@ __global__ void __launch_bounds__(32 + G * kSegGroupThreads + kSegMergeThreads, 
                     }
                 }
             }
-            // final flush into the group's shared accumulators.  Shared-memory atomics cost one pass per
-            // distinct address, which beats a shuffle tree per distinct label on fine-grained maps and is
-            // a single 32-way same-address pass on blocky ones.
-            // (fp32 shared-memory atomics are CAS loops: 128 threads on one address serialise 128 rounds.  The
-            // final flush is therefore aggregated per warp first — lanes holding the same running label are
-            // summed with shuffles and one lane adds — which on blocky maps is one or two rounds.)
-            const bool staged = p.flush_mode == 2 && dcount <= 32;
+            // final flush of the open runs into the group's accumulators: with <= 32 usable labels a staged gather
+            // (atomic-free and deterministic: the warp's totals per dense label, lane-ordered sums; the publishing
+            // thread below adds the four warps in warp order), above that one shared-memory atomic per lane (one pass
+            // per distinct address, which beats a shuffle tree per distinct label on fine-grained maps)
+            const bool staged = dcount <= 32;
             float* wt = c_wtot + (sparity * kSegGroupWarps + gw) * 64;
             if (staged) {
-                // atomic-free and deterministic: the warp's totals per dense label (lane-ordered sums); the
-                // publishing thread below adds the four warps in warp order
                 seg_warp_totals(reinterpret_cast<float2*>(wt), lane, cur, a1, a2);
-            } else if (p.flush_mode != 1) {
-                if (cur >= 0) {
-                    atomicAdd(&acc[cur * 2 + 0], a1);
-                    atomicAdd(&acc[cur * 2 + 1], a2);
-                }
-            } else {
-                unsigned pending = __ballot_sync(0xffffffffu, cur >= 0);
-                while (pending) {
-                    const int leader = __ffs(pending) - 1;
-                    const int lcur = __shfl_sync(0xffffffffu, cur, leader);
-                    const bool mine = cur == lcur;
-                    const float s1 = warp_sum(mine ? a1 : 0.f), s2 = warp_sum(mine ? a2 : 0.f);
-                    if (lane == leader) {
-                        atomicAdd(&acc[lcur * 2 + 0], s1);
-                        atomicAdd(&acc[lcur * 2 + 1], s2);
-                    }
-                    pending &= ~__ballot_sync(0xffffffffu, mine);
-                }
+            } else if (cur >= 0) {
+                atomicAdd(&acc[cur * 2 + 0], a1);
+                atomicAdd(&acc[cur * 2 + 1], a2);
             }
             named_bar_sync(1 + group, kSegGroupThreads);
             // publish: one self-validating 8-byte slot per usable label (no fence, no atomic, no counter)
@@ -1002,22 +978,22 @@ SegTmaLayout seg_tma_layout(int64_t n, int64_t c, int64_t hw_c, int64_t hw_s) {
     return l;
 }
 
-template <int G>
 int launch_seg_tma(const SegTmaParams& p, cudaStream_t st) {
     constexpr size_t stage = kSegStageBytes;
     constexpr size_t cache = kSegCacheBytes;
-    constexpr size_t smem = G * (kSegDepth * stage + cache) + G * kSegDepth * sizeof(SegDesc) + 2 * G * kSegDepth * sizeof(uint64_t) +
-                            2 * kSegMailbox * sizeof(uint64_t) + kSegMailbox * sizeof(int64_t) +
+    constexpr size_t smem = kSegGroups * (kSegDepth * stage + cache) + kSegGroups * kSegDepth * sizeof(SegDesc) +
+                            2 * kSegGroups * kSegDepth * sizeof(uint64_t) + 2 * kSegMailbox * sizeof(uint64_t) +
+                            kSegMailbox * sizeof(int64_t) +
                             kSegTicketBatch * sizeof(SegDecoded);
     static PerDeviceFlag configured_on;
     bool& configured = configured_on.get();
     if (!configured) {
-        RPST_CUDA(cudaFuncSetAttribute(seg_tma_kernel<G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        RPST_CUDA(cudaFuncSetAttribute(seg_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         configured = true;
     }
     int64_t grid = sm_count();
     if (grid > (int64_t)p.total_items) grid = p.total_items;
-    seg_tma_kernel<G><<<(int)grid, 32 + G * kSegGroupThreads + kSegMergeThreads, smem, st>>>(p);
+    seg_tma_kernel<<<(int)grid, 32 + kSegGroups * kSegGroupThreads + kSegMergeThreads, smem, st>>>(p);
     RPST_CUDA(cudaGetLastError());
     return RPST_OK;
 }
@@ -1143,11 +1119,10 @@ extern "C" int rpst_seg_adain_fwd(const float* content, const float* style, cons
         const int64_t planes = n * c;
         seg_shift_kernel<<<(unsigned)((planes * 2 * kLabels + 255) / 256), 256, 0, st>>>(q);
         RPST_CUDA(cudaGetLastError());
-        q.flush_mode = (int)g_knobs.seg_flush;
         const int64_t total = seg_plan_schedule(q, prev != nullptr);
         RPST_CHECK_ARG(total < (1ll << 31), "seg_adain: too many work items (%lld); split the call", (long long)total);
         q.total_items = (unsigned)total;
-        const int rc = g_knobs.seg_groups == 3 ? launch_seg_tma<3>(q, st) : launch_seg_tma<4>(q, st);   // 4 groups x 2 stages x 20 KiB
+        const int rc = launch_seg_tma(q, st);
         if (rc) return rc;
         // a sample with more than kMaxDense usable labels makes the slot kernel exit at once and the
         // register-staged kernel below run instead (device-side decision: no host synchronisation)

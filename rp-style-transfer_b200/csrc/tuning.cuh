@@ -12,17 +12,13 @@ struct Knobs {
     int64_t adain_big_lag_bytes = 128ll << 20;  // the same for planes >= 4 MiB: see plan_schedule
     int64_t adain_mvn_lag_bytes = 44ll << 20;   // the same for style == NULL (mean_variance_norm): see plan_schedule
     int64_t adain_hints = 1;                    // L2 eviction-priority hints on the streaming loads / stores
-    int64_t adain_ctas_per_sm = 4;              // persistent CTAs per SM of the register-staged pipelined kernel
     int64_t adain_path = 0;      // 0: TMA-staged kernel when alignment allows, 1: register-staged kernel; 1 also turns
                                  // off the segment AdaIN TMA kernel (seg.cu)
-    int64_t adain_stages = 6;    // TMA ring depth (32 KiB per stage)
     int64_t adain_twin_apply = 1;               // TMA kernel, no prev: apply items carry two content chunks (32 KiB per stage)
     int64_t adain_group_merge_min_spp = 512;    // see merge_plane_coef_group
     int64_t adain_merge_lead = 0;               // 0: lag / 2
     // segment AdaIN (seg.cu)
     int64_t seg_lag_bytes = 256ll << 20;  // content bytes between statistics and apply
-    int64_t seg_groups = 4;               // consumer groups (= stages) of the segment TMA kernel
-    int64_t seg_flush = 2;                // final flush: 0 shared atomics per lane, 1 warp-aggregated, 2 staged gather (atomic-free)
     // SANet attention (sanet.cu, flash.cu)
     int64_t attn_flash = 1;       // 1: C = 512 attention takes the single-kernel flash path when the shape allows
     int64_t attn_flash_prof = 0;  // device pointer to 32 x uint64 cycle counters (0 = off); bring-up / tuning only
@@ -34,8 +30,6 @@ struct Knobs {
     int64_t wct_roots_ns = 1;     // 1 Newton-Schulz roots with Jacobi for flagged matrices, 0 Jacobi only,
                                   // 2 Newton-Schulz but every matrix flagged (exercises the predicated path)
     int64_t ns_dmma = 1;          // 1 = fp64 tensor-core products (mma.sync f64) for even orders, 0 = DFMA kernel
-    int64_t eig_wide = -1;        // -1 auto, 0 / 1 force 16- / 32-column blocks, -2 auto + print cluster occupancy,
-                                  // 2 16-column blocks padded to one CTA per SM + print cluster occupancy
     // pointwise convolution (pwconv.cu)
     int64_t pw_x_tma = 1;  // 1 = x tiles by tensor-map TMA when the shape allows, 0 = register-staged converters
 };

@@ -114,7 +114,7 @@ def table_knobs():
 def test_knob_docs_match_table():
     documented = header_knobs()
     table = table_knobs()
-    assert len(table) == len(set(table)) >= 23
+    assert len(table) == len(set(table)) >= 18
     assert set(documented) == set(table), set(documented) ^ set(table)
     block = re.search(r"/\* Tuning knobs(.*?)\*/", open(HEADER).read(), flags=re.S).group(1)
     named = set(re.findall(r'^ \*\s+"(\w+)"', block, flags=re.M))
@@ -135,7 +135,7 @@ def test_knob_ranges_are_enforced(lib):
     """Both ends of each documented range are accepted; one step outside is rejected, names the knob, the range and
     the value, and leaves the knob as it was."""
     documented = header_knobs()
-    assert len(documented) >= 23
+    assert len(documented) >= 18
     for name, (lo, hi, _) in documented.items():
         key = name.encode()
         old = lib.rpst_get_tuning(key)
@@ -153,6 +153,19 @@ def test_knob_ranges_are_enforced(lib):
         finally:
             assert lib.rpst_set_tuning(key, old) == 0
         assert lib.rpst_get_tuning(key) == old, name
+
+
+RETIRED_KNOBS = ("adain_stages", "adain_ctas_per_sm", "seg_groups", "seg_flush", "eig_wide")
+
+
+def test_retired_knobs_are_unknown(lib):
+    """Knobs that once picked kernel instantiations no input reaches are gone: setting one fails as an unknown name,
+    and reading one returns -1."""
+    for name in RETIRED_KNOBS:
+        key = name.encode()
+        assert lib.rpst_set_tuning(key, 0) == -1, name
+        assert f"unknown tuning knob '{name}'".encode() in lib.rpst_last_error(), lib.rpst_last_error()
+        assert lib.rpst_get_tuning(key) == -1, name
 
 
 def test_read_only_knob_is_rejected(lib):

@@ -1,5 +1,5 @@
-"""Batched 256x256 matrix square roots: 16-column blocks (8-CTA clusters) vs 32-column blocks (4-CTA clusters), with the
-cluster occupancy the driver reports.  GPU box only."""
+"""Batched 256x256 matrix square roots at the automatic Jacobi block width: 16-column blocks (8-CTA clusters) up to
+batch 20, 32-column blocks (4-CTA clusters) above.  GPU box only."""
 import json, os, sys, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import rpst
@@ -16,14 +16,5 @@ for batch in (1, 8, 12, 16, 32):
     g = torch.Generator(device="cuda").manual_seed(n)
     a = torch.randn(batch, n, 2 * n, device="cuda", dtype=torch.float64, generator=g)
     a = a @ a.transpose(1, 2) / (2 * n)
-    row = {"batch": batch}
-    for wide, name in ((0, "bc16"), (2, "bc16_one_cta_per_sm"), (1, "bc32")):
-        rpst.set_tuning("eig_wide", wide)
-        row["ms_" + name] = round(t(lambda: rpst.matrix_sqrt(a), 2 if wide == 2 else 5), 3)
-    print(json.dumps(row), flush=True)
-rpst.set_tuning("eig_wide", -2)
-a = torch.randn(16, n, 2 * n, device="cuda", dtype=torch.float64)
-a = a @ a.transpose(1, 2) / (2 * n)
-rpst.matrix_sqrt(a)
-torch.cuda.synchronize()
-rpst.set_tuning("eig_wide", -1)
+    print(json.dumps({"batch": batch, "block_cols": 32 if batch * (n // 32) > 160 else 16,
+                      "ms": round(t(lambda: rpst.matrix_sqrt(a)), 3)}), flush=True)

@@ -57,13 +57,12 @@ print(json.dumps({"torch_copy_GBs": 2 * E * 10 / (a.elapsed_time(b) / 1e3) / 1e9
 del x
 
 rows = []
-for lag_mb, hints, ctas in itertools.product([24, 32, 48, 64], [1, 0], [5, 6]):
+for lag_mb, hints in itertools.product([24, 32, 48, 64], [1, 0]):
     rpst.set_tuning("adain_lag_bytes", lag_mb << 20)
     rpst.set_tuning("adain_hints", hints)
-    rpst.set_tuning("adain_stages", ctas)
     t_plain = timeit(None)
     t_blend = timeit(p)
-    row = {"lag_mb": lag_mb, "hints": hints, "stages": ctas, "plain_ms": round(t_plain, 4),
+    row = {"lag_mb": lag_mb, "hints": hints, "plain_ms": round(t_plain, 4),
            "plain_GBs": round(3 * E / (t_plain / 1e3) / 1e9, 1), "blend_ms": round(t_blend, 4),
            "blend_GBs": round(4 * E / (t_blend / 1e3) / 1e9, 1)}
     rows.append(row)
