@@ -64,7 +64,7 @@ RPST_API const char* rpst_last_error(void);
  *                                                        by a whole warp group instead of one warp
  *   "adain_merge_lead"          0..INT64_MAX  0          TMA kernel: planes between a plane's merge and its first apply, clamped
  *                                                        to 1..lag-1; 0: lag / 2
- * Segment AdaIN, TMA kernel (rpst_seg_adain_fwd):
+ * Segment AdaIN, TMA kernel (rpst_seg_adain_fwd, rpst_seg_adain_fwd_mapped):
  *   "seg_lag_bytes"             0..INT64_MAX  268435456  content bytes between a plane's statistics and its apply (256 MiB)
  * SANet attention (rpst_sanet_attn_fwd):
  *   "attn_flash"                0..1          1          1: C = 512 attention runs as one flash-style kernel when the shape
@@ -193,6 +193,21 @@ RPST_API int rpst_seg_adain_fwd(const float* content, const float* style, const 
                        const uint8_t* s_labels, const float* prev, float* out, int64_t n, int64_t c,
                        int64_t hw_c, int64_t hw_s, float eps, int32_t* label_info, void* workspace,
                        size_t workspace_bytes, void* stream);
+
+/* Same as rpst_seg_adain_fwd, with plane maps and a strided output, as rpst_adain_fwd_mapped adds to
+ * rpst_adain_fwd, so the masked decodes neither gather shuffled / sorted features nor concatenate copies:
+ *   output plane p = i*c + ch reads its content from plane content_map[p] and its style from plane
+ *   style_map[p] of the SAME tensors (global plane indices in [0, n*c); either map may be NULL = identity);
+ *   the label maps, the validity rule and label_info belong to the OUTPUT sample i (c_labels[i],
+ *   s_labels[i]), as they would for the gathered tensors; prev [n,c,hw_c] is indexed by the output plane;
+ *   plane (i, ch) of out is written at out + i*out_batch_stride + ch*hw_c (out_batch_stride >= c*hw_c;
+ *   (c_prev + c)*hw_c writes the channel slice of cat([prev_feats, seg-AdaIN], 1)).
+ * Workspace: rpst_seg_adain_workspace_bytes.  n*c must be < 2^31. */
+RPST_API int rpst_seg_adain_fwd_mapped(const float* content, const float* style, const uint8_t* c_labels,
+                              const uint8_t* s_labels, const float* prev, float* out, int64_t n, int64_t c,
+                              int64_t hw_c, int64_t hw_s, int64_t out_batch_stride, float eps,
+                              const int32_t* content_map, const int32_t* style_map, int32_t* label_info,
+                              void* workspace, size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * a12 cal_dist(A, B)                                                  network/base.py:349-360

@@ -14,7 +14,8 @@ from .mrf import MRFLoss, cal_affinity_map, cal_dist, mrf_match, packed_gemm
 from .wct import matrix_inv_sqrt, matrix_sqrt, spd_roots, wct_fuse, whiten_and_color
 from .sanet import (AdaptiveSANet, AdaptiveTransform, AEALReluModule, AEAModule, SANet, Transform, attention_core,
                     cal_affinity_matrix)
-from .segment import adaptive_instance_normalization_with_segment, do_mask_stylized, load_label_map, seg_adain_batch
+from .segment import (adaptive_instance_normalization_with_segment, do_mask_stylized, load_label_map, seg_adain_batch,
+                      seg_adain_concat)
 
 from .conv import adain_from_stats, conv1x1
 from .decode import multiscale_transform

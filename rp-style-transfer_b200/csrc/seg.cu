@@ -30,9 +30,11 @@ struct SegParams {
     const float* style;
     const uint8_t* c_lab;   // [n, hw_c]
     const uint8_t* s_lab;   // [n, hw_s]
-    const float* prev;      // may be null
-    float* out;
-    int64_t n, channels, hw_c, hw_s;
+    const float* prev;      // may be null; indexed by the output plane
+    float* out;             // plane (i, ch) at out + i*out_batch_stride + ch*hw_c
+    const int* cmap;        // source plane of content / style per output plane (null: identity)
+    const int* smap;
+    int64_t n, channels, hw_c, hw_s, out_batch_stride;
     float eps;
     int hints;
     int ipp_c, ipp_s, lag;
@@ -74,6 +76,12 @@ __global__ void __launch_bounds__(256) seg_hist_kernel(const uint8_t* __restrict
         atomicAdd(&cnt[slot], h[threadIdx.x]);
         atomicMin(&first[slot], f[threadIdx.x]);
     }
+}
+
+// plane maps (rpst_seg_adain_fwd_mapped): output plane -> plane of the content / style tensor that feeds it.
+// Everything else (labels, validity, slots, coefficients, prev) stays indexed by the output plane.
+__device__ __forceinline__ int64_t src_plane(const int* map, int64_t plane) {
+    return map ? (int64_t)__ldg(map + plane) : plane;
 }
 
 __device__ __forceinline__ bool label_usable(int nc, int ns) {
@@ -157,7 +165,7 @@ __global__ void __launch_bounds__(kPipeThreads, 3) seg_pipe_kernel(SegParams p) 
             // ------------------------------------------------ statistics item (content or style)
             const bool is_style = it.kind == 1;
             const int64_t hw = is_style ? p.hw_s : p.hw_c;
-            const float* x = (is_style ? p.style : p.content) + it.plane * hw;
+            const float* x = is_style ? p.style + src_plane(p.smap, it.plane) * hw : p.content + src_plane(p.cmap, it.plane) * hw;
             const uint8_t* labels = (is_style ? p.s_lab : p.c_lab) + sample * hw;
             const int* first = p.first + (sample * 2 + it.kind) * kLabels;
             const int64_t e0 = (int64_t)it.chunk * CHUNK;
@@ -244,8 +252,8 @@ __global__ void __launch_bounds__(kPipeThreads, 3) seg_pipe_kernel(SegParams p) 
                 const int nc = __ldg(cnt_c + l), ns = __ldg(cnt_s + l);
                 float4 cf = make_float4(0.f, 1.f, 0.f, 0.f);  // identity for unusable labels
                 if (label_usable(nc, ns)) {
-                    const float kc = __ldg(p.content + it.plane * p.hw_c + __ldg(p.first + (sample * 2 + 0) * kLabels + l));
-                    const float ks = __ldg(p.style + it.plane * p.hw_s + __ldg(p.first + (sample * 2 + 1) * kLabels + l));
+                    const float kc = __ldg(p.content + src_plane(p.cmap, it.plane) * p.hw_c + __ldg(p.first + (sample * 2 + 0) * kLabels + l));
+                    const float ks = __ldg(p.style + src_plane(p.smap, it.plane) * p.hw_s + __ldg(p.first + (sample * 2 + 1) * kLabels + l));
                     const float2 gc = __ldcg(p.gsum + (it.plane * 2 + 0) * kLabels + l);
                     const float2 gs = __ldcg(p.gsum + (it.plane * 2 + 1) * kLabels + l);
                     const float fnc = (float)nc, fns = (float)ns;
@@ -267,9 +275,9 @@ __global__ void __launch_bounds__(kPipeThreads, 3) seg_pipe_kernel(SegParams p) 
             const int64_t e0 = (int64_t)it.chunk * CHUNK;
             const int64_t rem = p.hw_c - e0;
             const int nvec = (int)((rem < CHUNK ? rem : CHUNK) / VEC);
-            const float* cbase = p.content + it.plane * p.hw_c + e0;
+            const float* cbase = p.content + src_plane(p.cmap, it.plane) * p.hw_c + e0;
             const float* pbase = p.prev ? p.prev + it.plane * p.hw_c + e0 : nullptr;
-            float* obase = p.out + it.plane * p.hw_c + e0;
+            float* obase = p.out + sample * p.out_batch_stride + (it.plane - sample * p.channels) * p.hw_c + e0;
             const uint8_t* labels = p.c_lab + sample * p.hw_c + e0;
             float c[kBatch][VEC], pv[kBatch][VEC];
             load_batch<VEC, T>(c, cbase, 0, nvec, pol_first, hint);
@@ -353,9 +361,11 @@ struct SegTmaParams {
     const float* style;
     const uint8_t* c_lab;
     const uint8_t* s_lab;
-    const float* prev;
-    float* out;
-    int64_t n, channels, hw_c, hw_s;
+    const float* prev;           // indexed by the output plane
+    float* out;                  // plane (i, ch) at out + i*out_batch_stride + ch*hw_c
+    const int* cmap;             // source plane of content / style per output plane (null: identity)
+    const int* smap;
+    int64_t n, channels, hw_c, hw_s, out_batch_stride;
     float eps;
     int ic, is, lag;             // content / style statistics chunks per plane, statistics lead in planes
     int ia, apply_elems;         // apply chunks per plane and their size (kSegHalfElems with prev, else kSegItemElems)
@@ -420,8 +430,8 @@ __global__ void seg_shift_kernel(SegTmaParams p) {
     const int slot = (int)((sample * 2 + which) * kLabels + l);
     float v = 0.f;
     if (p.cnt[slot] > 0) {
-        const int64_t hw = which ? p.hw_s : p.hw_c;
-        v = (which ? p.style : p.content)[plane * hw + p.first[slot]];
+        v = which ? p.style[src_plane(p.smap, plane) * p.hw_s + p.first[slot]]
+                  : p.content[src_plane(p.cmap, plane) * p.hw_c + p.first[slot]];
     }
     p.shift[idx] = v;
 }
@@ -560,12 +570,15 @@ __global__ void __launch_bounds__(32 + kSegGroups * kSegGroupThreads + kSegMerge
             // capped both TMA kernels at ~1.3 M items/s per SM).
             static_assert(kSegGroups * kSegDepth >= kSegTicketBatch, "a batch must not reuse a stage");
             int kind = 3, chunk = 0;    // lanes >= batch: treated like a merge (skipped)
-            int64_t plane = 0;
+            int64_t plane = 0, splane = 0;   // output plane; source plane of the tensor the item streams
             if (lane < kSegTicketBatch) {
                 kind = -1;
                 const unsigned t = base + (unsigned)lane;
                 if (t < p.total_items) seg_decode(t, p, kind, plane, chunk);
                 dec[lane].kind = kind; dec[lane].chunk = chunk; dec[lane].plane = plane;
+                // the lane that decodes a ticket also issues it: the map load overlaps the empty-stage wait below
+                if (kind == 1) splane = src_plane(p.smap, plane);
+                else if (kind == 0 || kind == 2) splane = src_plane(p.cmap, plane);
             }
             __syncwarp();
             const unsigned stopmask = __ballot_sync(0xffffffffu, kind < 0);
@@ -603,7 +616,7 @@ __global__ void __launch_bounds__(32 + kSegGroups * kSegGroupThreads + kSegMerge
                 const uint32_t bytes = (uint32_t)nvec * 16u;
                 unsigned char* st = stages + (size_t)stage * STAGE_BYTES;
                 const int64_t sample = (int)plane / (int)p.channels;
-                const float* src = (is_style ? p.style : p.content) + plane * hw + e0;
+                const float* src = (is_style ? p.style : p.content) + splane * hw + e0;
                 const uint8_t* lab = (is_style ? p.s_lab : p.c_lab) + sample * hw + e0;
                 const bool has_prev = kind == 2 && p.prev != nullptr;
                 mbar_arrive_expect_tx(&full[stage], bytes + (has_prev ? bytes : 0u) + (uint32_t)nvec * 4u);
@@ -876,7 +889,8 @@ __global__ void __launch_bounds__(32 + kSegGroups * kSegGroupThreads + kSegMerge
                 cached_apply = plane;
             }
             const bool has_prev = p.prev != nullptr;
-            float4* o4 = reinterpret_cast<float4*>(p.out + plane * p.hw_c + (int64_t)chunk * p.apply_elems) + gw * warp_vecs;
+            float4* o4 = reinterpret_cast<float4*>(p.out + sample * p.out_batch_stride + (plane - sample * p.channels) * p.hw_c +
+                                                   (int64_t)chunk * p.apply_elems) + gw * warp_vecs;
             uint32_t last_w = 0;
             float4 cf = c_coef[kMaxDense];
             bool have = false;
@@ -1060,15 +1074,43 @@ extern "C" size_t rpst_seg_adain_workspace_bytes(int64_t n, int64_t c, int64_t h
 
 }
 
+namespace {
+int seg_adain_fwd_impl(const float* content, const float* style, const uint8_t* c_labels, const uint8_t* s_labels,
+                       const float* prev, float* out, int64_t n, int64_t c, int64_t hw_c, int64_t hw_s,
+                       int64_t out_batch_stride, float eps, const int* content_map, const int* style_map,
+                       int32_t* label_info, void* workspace, size_t workspace_bytes, void* stream);
+}
+
 extern "C" int rpst_seg_adain_fwd(const float* content, const float* style, const uint8_t* c_labels,
                                   const uint8_t* s_labels, const float* prev, float* out, int64_t n, int64_t c,
                                   int64_t hw_c, int64_t hw_s, float eps, int32_t* label_info, void* workspace,
                                   size_t workspace_bytes, void* stream) {
+    return seg_adain_fwd_impl(content, style, c_labels, s_labels, prev, out, n, c, hw_c, hw_s, c * hw_c, eps, nullptr,
+                              nullptr, label_info, workspace, workspace_bytes, stream);
+}
+
+extern "C" int rpst_seg_adain_fwd_mapped(const float* content, const float* style, const uint8_t* c_labels,
+                                         const uint8_t* s_labels, const float* prev, float* out, int64_t n, int64_t c,
+                                         int64_t hw_c, int64_t hw_s, int64_t out_batch_stride, float eps,
+                                         const int32_t* content_map, const int32_t* style_map, int32_t* label_info,
+                                         void* workspace, size_t workspace_bytes, void* stream) {
+    RPST_CHECK_ARG(n * c < (1ll << 31), "seg_adain_mapped: plane index does not fit int32");
+    return seg_adain_fwd_impl(content, style, c_labels, s_labels, prev, out, n, c, hw_c, hw_s, out_batch_stride, eps,
+                              content_map, style_map, label_info, workspace, workspace_bytes, stream);
+}
+
+namespace {
+int seg_adain_fwd_impl(const float* content, const float* style, const uint8_t* c_labels, const uint8_t* s_labels,
+                       const float* prev, float* out, int64_t n, int64_t c, int64_t hw_c, int64_t hw_s,
+                       int64_t out_batch_stride, float eps, const int* content_map, const int* style_map,
+                       int32_t* label_info, void* workspace, size_t workspace_bytes, void* stream) {
     RPST_CHECK_ARG(n >= 0 && c >= 0 && hw_c >= 0 && hw_s >= 0, "seg_adain: negative size");
     if (n == 0 || c == 0 || hw_c == 0) return RPST_OK;
     RPST_CHECK_ARG(content && style && c_labels && s_labels && out, "seg_adain: null pointer");
     RPST_CHECK_ARG(hw_s > 0, "seg_adain: empty style map");
     RPST_CHECK_ARG(hw_c < (1ll << 31) && hw_s < (1ll << 31), "seg_adain: plane too large");
+    RPST_CHECK_ARG(out_batch_stride >= c * hw_c, "seg_adain: out_batch_stride (%lld) < c*hw_c (%lld)",
+                   (long long)out_batch_stride, (long long)(c * hw_c));
     RPST_CHECK_ARG(out != content && out != style && out != prev, "seg_adain: out must not alias an input");
     const size_t need = rpst_seg_adain_workspace_bytes(n, c, hw_c, hw_s);
     if (workspace == nullptr || workspace_bytes < need) {
@@ -1082,14 +1124,15 @@ extern "C" int rpst_seg_adain_fwd(const float* content, const float* style, cons
     int hist_blocks0 = (int)((hw_max0 + 16383) / 16384);
     if (hist_blocks0 > 256) hist_blocks0 = 256;
     const bool tma_ok = g_knobs.adain_path == 0 && hw_c % 16 == 0 && hw_s % 16 == 0 &&
-                        aligned(content, 16) && aligned(style, 16) && aligned(out, 16) && (!prev || aligned(prev, 16)) &&
-                        aligned(c_labels, 16) && aligned(s_labels, 16);
+                        aligned(content, 16) && aligned(style, 16) && aligned(out, 16) && out_batch_stride % 4 == 0 &&
+                        (!prev || aligned(prev, 16)) && aligned(c_labels, 16) && aligned(s_labels, 16);
     const int* run_flag = nullptr;
     if (tma_ok) {
         const SegTmaLayout t = seg_tma_layout(n, c, hw_c, hw_s);
         SegTmaParams q{};
         q.content = content; q.style = style; q.c_lab = c_labels; q.s_lab = s_labels; q.prev = prev; q.out = out;
-        q.n = n; q.channels = c; q.hw_c = hw_c; q.hw_s = hw_s; q.eps = eps;
+        q.cmap = content_map; q.smap = style_map;
+        q.n = n; q.channels = c; q.hw_c = hw_c; q.hw_s = hw_s; q.out_batch_stride = out_batch_stride; q.eps = eps;
         q.ticket = reinterpret_cast<unsigned*>(base + t.ticket);
         q.ready = reinterpret_cast<int*>(base + t.ready);
         int* cnt = reinterpret_cast<int*>(base + t.cnt);
@@ -1132,7 +1175,8 @@ extern "C" int rpst_seg_adain_fwd(const float* content, const float* style, cons
     const SegLayout l = seg_layout(n, c);
     SegParams p{};
     p.content = content; p.style = style; p.c_lab = c_labels; p.s_lab = s_labels; p.prev = prev; p.out = out;
-    p.n = n; p.channels = c; p.hw_c = hw_c; p.hw_s = hw_s; p.eps = eps;
+    p.cmap = content_map; p.smap = style_map;
+    p.n = n; p.channels = c; p.hw_c = hw_c; p.hw_s = hw_s; p.out_batch_stride = out_batch_stride; p.eps = eps;
     p.hints = (int)g_knobs.adain_hints;
     p.ticket = reinterpret_cast<unsigned*>(base);
     p.done = reinterpret_cast<int*>(base + l.done_off);
@@ -1157,7 +1201,7 @@ extern "C" int rpst_seg_adain_fwd(const float* content, const float* style, cons
     }
 
     const bool vec = hw_c % 4 == 0 && hw_s % 4 == 0 && aligned(content, 16) && aligned(style, 16) && aligned(out, 16) &&
-                     (!prev || aligned(prev, 16)) && aligned(c_labels, 4) && aligned(s_labels, 4);
+                     out_batch_stride % 4 == 0 && (!prev || aligned(prev, 16)) && aligned(c_labels, 4) && aligned(s_labels, 4);
     const int64_t chunk = (int64_t)kPipeThreads * kPerThread * (vec ? 4 : 1);
     p.ipp_c = (int)((hw_c + chunk - 1) / chunk);
     p.ipp_s = (int)((hw_s + chunk - 1) / chunk);
@@ -1176,5 +1220,6 @@ extern "C" int rpst_seg_adain_fwd(const float* content, const float* style, cons
     RPST_CUDA(cudaGetLastError());
     return RPST_OK;
 }
+}  // namespace
 
 RPST_WATCHDOG_SETTER(seg)

@@ -24,32 +24,25 @@ def multiscale_transform(content_feats: Sequence[torch.Tensor], style_feats: Seq
     return outs
 
 
-def _gather(feat, plane_map):
-    return feat if plane_map is None else feat.flatten(0, 1)[plane_map.long()].view_as(feat)
-
-
 def decode_multiscale(self, content_feats, style_feats, use_mask=False, c_mask_path=None, s_mask_path=None,
                       plane_maps=None):
     """MultiScaleAdaINRPNet.decode (network/adain_rp.py:286-302): top level plain (seg-)AdaIN, every
     shallower level `decoder(prev + (seg-)AdaIN(c_l, s_l))` with the add fused into the transform.
     `sort_by_weights` (:230-249, applied here when `self._sort`) and the channel `shuffle` of `test()`
     (:256-260, handed over as `plane_maps` by `test_multiscale`) become plane maps of the kernel call
-    instead of permuted copies.  Like the reference, content and style are sorted by the SAME attention
-    weights (the ones the shared encoder stored last)."""
+    instead of permuted copies, in the masked (segment AdaIN) branch too.  Like the reference, content and
+    style are sorted by the SAME attention weights (the ones the shared encoder stored last)."""
     levels = len(content_feats)
     maps = list(plane_maps) if plane_maps is not None else [None] * levels
     if self._sort:
         for idx, enc in enumerate(self.rp_shared_encoder):
             maps[idx] = F.compose_maps(maps[idx], F.sort_map(enc.attention_map))
-    if use_mask:   # the segment op takes dense tensors: materialise the permutation for it
-        content_feats = [_gather(c, m) for c, m in zip(content_feats, maps)]
-        style_feats = [_gather(s, m) for s, m in zip(style_feats, maps)]
-        maps = [None] * levels
 
     def level(l, prev):
         cf, sf = content_feats[l], style_feats[l]
         if use_mask:
-            return SEG.do_mask_stylized(cf, sf, c_mask_path, s_mask_path, prev=prev)
+            return SEG.do_mask_stylized(cf, sf, c_mask_path, s_mask_path, prev=prev, content_map=maps[l],
+                                        style_map=maps[l])
         if maps[l] is not None:
             return F.adain_mapped(cf, sf, maps[l], maps[l], prev=prev)
         return F.adaptive_instance_normalization(cf, sf) if prev is None else F.adain_blend(prev, cf, sf)
@@ -112,12 +105,15 @@ def decode_ldms(self, content_feats, style_feats, use_mask=False, c_mask_path=No
 
 def decode_ld_concat(self, content_feats, style_feats, use_mask=False, c_mask_path=None, s_mask_path=None):
     """LDMSAdaINRPNet4.decode (network/adain_rp.py:780-799, inherited by LDMS 5):
-    `cat([stylized, AdaIN(c_l, s_l)], 1)` with the AdaIN half written straight into the result."""
+    `cat([stylized, (seg-)AdaIN(c_l, s_l)], 1)` with the AdaIN half written straight into the result."""
     stylized = self.rp_dec0(_top(self, content_feats, style_feats, use_mask, c_mask_path, s_mask_path))
     lower = list(zip(content_feats[:-1], style_feats[:-1]))[::-1]
     for i, (cf, sf) in enumerate(lower):
         if use_mask:
-            fused = torch.cat([stylized, SEG.do_mask_stylized(cf, sf, c_mask_path, s_mask_path)], dim=1)
+            hc, wc = cf.shape[2:]
+            hs, ws = sf.shape[2:]
+            fused = SEG.seg_adain_concat(stylized, cf, sf, SEG.stack_label_maps(c_mask_path, wc, hc, cf.device),
+                                         SEG.stack_label_maps(s_mask_path, ws, hs, sf.device))
         else:
             fused = F.adain_concat(stylized, cf, sf)
         stylized = getattr(self, f'rp_dec{i + 1}')(fused)

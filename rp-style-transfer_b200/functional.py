@@ -293,6 +293,15 @@ def compose_maps(first: Optional[torch.Tensor], then: Optional[torch.Tensor]) ->
     return first[then.long()].contiguous()
 
 
+def _check_map(m: Optional[torch.Tensor], name: str, planes: int) -> Optional[torch.Tensor]:
+    """A plane map argument: None (identity) or a CUDA int32 tensor with one entry per output plane."""
+    if m is None:
+        return None
+    if not m.is_cuda or m.dtype != torch.int32 or m.numel() != planes:
+        raise TypeError(f"rpst: `{name}` must be a CUDA int32 tensor with N*C = {planes} entries")
+    return m.contiguous()
+
+
 @device_guard
 def adain_mapped(content_feat: torch.Tensor, style_feat: torch.Tensor, content_map: Optional[torch.Tensor] = None,
                  style_map: Optional[torch.Tensor] = None, prev: Optional[torch.Tensor] = None) -> torch.Tensor:
@@ -304,15 +313,7 @@ def adain_mapped(content_feat: torch.Tensor, style_feat: torch.Tensor, content_m
     p = None if prev is None else _prep(prev, "prev")
     n, ch = c.shape[:2]
     hw = c[0, 0].numel() if c.numel() else 0
-
-    def chk(m, name):
-        if m is None:
-            return None
-        if not m.is_cuda or m.dtype != torch.int32 or m.numel() != n * ch:
-            raise TypeError(f"rpst: `{name}` must be a CUDA int32 tensor with N*C = {n * ch} entries")
-        return m.contiguous()
-
-    cm, sm = chk(content_map, "content_map"), chk(style_map, "style_map")
+    cm, sm = _check_map(content_map, "content_map", n * ch), _check_map(style_map, "style_map", n * ch)
     if _needs_grad(c, s, p):
         # training: gather through autograd, then the differentiable kernel path
         cg = c if cm is None else c.flatten(0, 1)[cm.long()].view_as(c)
