@@ -53,6 +53,22 @@ __device__ __forceinline__ bool watchdog_expired(uint64_t t0) {
     }                                                                                                        \
     }
 
+// Global-memory spin wait on a value the caller has loaded once already: while `ready()` says it is not ready, back off
+// `sleep_ns`, `reload()` it and trap once the watchdog expires.  A value that is ready at once costs no timer read, no
+// sleep and no load.  A reload that finds the value ready returns at once: the watchdog (a load of its limit and a
+// timer read) is looked at only on the way back to sleep.
+template <class Reload, class Ready>
+__device__ __forceinline__ void spin_wait(unsigned sleep_ns, Reload reload, Ready ready) {
+    if (ready()) return;
+    const uint64_t t0 = global_timer_ns();
+    for (;;) {
+        __nanosleep(sleep_ns);
+        reload();
+        if (ready()) return;
+        if (watchdog_expired(t0)) __trap();
+    }
+}
+
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
     if (mbar_try_wait(bar, parity)) return;
     const uint64_t t0 = global_timer_ns();

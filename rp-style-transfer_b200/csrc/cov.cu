@@ -254,11 +254,8 @@ __device__ __forceinline__ void grid_barrier(int* counter, int k) {
     if (threadIdx.x == 0) {
         atomicAdd(counter, 1);
         const int target = k * (int)gridDim.x;
-        const uint64_t t0 = global_timer_ns();
-        while (ld_acquire(counter) < target) {
-            __nanosleep(32);
-            if (watchdog_expired(t0)) __trap();
-        }
+        int arrived = ld_acquire(counter);
+        spin_wait(32, [&] { arrived = ld_acquire(counter); }, [&] { return arrived >= target; });
     }
     __syncthreads();
 }

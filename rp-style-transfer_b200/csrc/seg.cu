@@ -89,38 +89,6 @@ __device__ __forceinline__ bool label_usable(int nc, int ns) {
     return nc > 10 && ns > 10 && (int64_t)nc < 100ll * ns && (int64_t)ns < 100ll * nc;
 }
 
-struct SegItem {
-    int kind;  // 0 content statistics, 1 style statistics, 2 apply
-    int64_t plane;
-    int chunk;
-};
-
-__device__ __forceinline__ SegItem seg_decode(unsigned t, const SegParams& p) {
-    const int64_t planes = p.n * p.channels;
-    const int64_t st = p.ipp_c + p.ipp_s;  // statistics items per plane
-    const int64_t lag = p.lag < planes ? p.lag : planes;
-    SegItem it;
-    int64_t tt = t;
-    auto stats = [&](int64_t plane, int64_t u) {
-        it.plane = plane;
-        if (u < p.ipp_c) { it.kind = 0; it.chunk = (int)u; }
-        else { it.kind = 1; it.chunk = (int)(u - p.ipp_c); }
-    };
-    if (tt < lag * st) { stats(tt / st, tt % st); return it; }
-    tt -= lag * st;
-    const int64_t round = st + p.ipp_c;
-    const int64_t steady = (planes - lag) * round;
-    if (tt < steady) {
-        int64_t r = tt / round, u = tt % round;
-        if (u < st) stats(r + lag, u);
-        else { it.kind = 2; it.plane = r; it.chunk = (int)(u - st); }
-        return it;
-    }
-    tt -= steady;
-    it.kind = 2; it.plane = (planes - lag) + tt / p.ipp_c; it.chunk = (int)(tt % p.ipp_c);
-    return it;
-}
-
 template <int VEC>
 __device__ __forceinline__ void load_labels(int (&lab)[VEC], const uint8_t* p) {
     if constexpr (VEC == 4) {
@@ -148,6 +116,7 @@ __global__ void __launch_bounds__(kPipeThreads, 3) seg_pipe_kernel(SegParams p) 
     const bool hint = p.hints != 0;
     const int lane = threadIdx.x & 31;
     if (p.run_flag != nullptr && __ldg(p.run_flag) == 0) return;
+    const unsigned planes = (unsigned)(p.n * p.channels);
 
     if (threadIdx.x == 0) s_ticket = atomicAdd(p.ticket, 1u);
     __syncthreads();
@@ -156,19 +125,21 @@ __global__ void __launch_bounds__(kPipeThreads, 3) seg_pipe_kernel(SegParams p) 
     while (t < p.total_items) {
         unsigned next = 0;
         if (threadIdx.x == 0) next = atomicAdd(p.ticket, 1u);
-        const SegItem it = seg_decode(t, p);
+        // a plane's statistics items are its content chunks, then its style chunks
+        const LagItem it = decode_lag(t, planes, (unsigned)p.lag, (unsigned)(p.ipp_c + p.ipp_s), (unsigned)p.ipp_c);
         const int64_t sample = it.plane / p.channels;
         const int* cnt_c = p.cnt + (sample * 2 + 0) * kLabels;
         const int* cnt_s = p.cnt + (sample * 2 + 1) * kLabels;
 
-        if (it.kind < 2) {
+        if (it.kind == 0) {
             // ------------------------------------------------ statistics item (content or style)
-            const bool is_style = it.kind == 1;
+            const int which = it.chunk >= p.ipp_c;   // 0 content, 1 style
+            const bool is_style = which == 1;
             const int64_t hw = is_style ? p.hw_s : p.hw_c;
             const float* x = is_style ? p.style + src_plane(p.smap, it.plane) * hw : p.content + src_plane(p.cmap, it.plane) * hw;
             const uint8_t* labels = (is_style ? p.s_lab : p.c_lab) + sample * hw;
-            const int* first = p.first + (sample * 2 + it.kind) * kLabels;
-            const int64_t e0 = (int64_t)it.chunk * CHUNK;
+            const int* first = p.first + (sample * 2 + which) * kLabels;
+            const int64_t e0 = (int64_t)(is_style ? it.chunk - p.ipp_c : it.chunk) * CHUNK;
             const int64_t rem = hw - e0;
             const int nvec = (int)((rem < CHUNK ? rem : CHUNK) / VEC);
             {
@@ -233,19 +204,14 @@ __global__ void __launch_bounds__(kPipeThreads, 3) seg_pipe_kernel(SegParams p) 
                 const int l = threadIdx.x;
                 const float r1 = s_acc[l][0], r2 = s_acc[l][1];
                 if (r1 != 0.f || r2 != 0.f) {
-                    float2* g = p.gsum + (it.plane * 2 + it.kind) * kLabels + l;
+                    float2* g = p.gsum + (it.plane * 2 + which) * kLabels + l;
                     atomicAdd(&g->x, r1);
                     atomicAdd(&g->y, r2);
                 }
             }
             __threadfence();
             __syncthreads();
-            if (threadIdx.x == 0) {
-                int old = atomicAdd(&p.done[it.plane], 1);
-                s_last = (old == p.ipp_c + p.ipp_s - 1);
-            }
-            __syncthreads();
-            if (s_last) {
+            if (gate_arrive(&p.done[it.plane], p.ipp_c + p.ipp_s, s_last)) {
                 // last statistics item of the plane: turn the sums into per-label AdaIN coefficients
                 __threadfence();
                 const int l = threadIdx.x;
@@ -268,7 +234,7 @@ __global__ void __launch_bounds__(kPipeThreads, 3) seg_pipe_kernel(SegParams p) 
                 __stcg(&p.coef[it.plane * kLabels + l], cf);
                 __threadfence();
                 __syncthreads();
-                if (threadIdx.x == 0) st_release(&p.ready[it.plane], 1);
+                if (threadIdx.x == 0) gate_publish(&p.ready[it.plane]);
             }
         } else {
             // ------------------------------------------------ apply item
@@ -282,9 +248,7 @@ __global__ void __launch_bounds__(kPipeThreads, 3) seg_pipe_kernel(SegParams p) 
             float c[kBatch][VEC], pv[kBatch][VEC];
             load_batch<VEC, T>(c, cbase, 0, nvec, pol_first, hint);
             if (pbase) load_batch<VEC, T>(pv, pbase, 0, nvec, pol_first, hint);
-            if (threadIdx.x == 0) {
-                while (ld_acquire(&p.ready[it.plane]) == 0) __nanosleep(100);
-            }
+            if (threadIdx.x == 0) gate_wait(&p.ready[it.plane]);
             __syncthreads();
             s_coef[threadIdx.x] = __ldcg(&p.coef[it.plane * kLabels + threadIdx.x]);
             __syncthreads();
@@ -457,7 +421,7 @@ __device__ __forceinline__ float canon_f(float v) {
     return __float_as_uint(v) == 0xffffffffu ? __uint_as_float(0x7fc00000u) : v;
 }
 
-__device__ __forceinline__ void seg_decode(unsigned t, const SegTmaParams& p, int& kind, int64_t& plane, int& chunk) {
+__device__ __forceinline__ void seg_tma_decode(unsigned t, const SegTmaParams& p, int& kind, int64_t& plane, int& chunk) {
     // the merge of a plane follows its statistics by one plane; the apply trails by L planes
     const unsigned P = (unsigned)(p.n * p.channels), L = (unsigned)p.lag, Lm = L - 1;
     const unsigned Ic = (unsigned)p.ic, St = (unsigned)(p.ic + p.is), Ia = (unsigned)p.ia;
@@ -574,7 +538,7 @@ __global__ void __launch_bounds__(32 + kSegGroups * kSegGroupThreads + kSegMerge
             if (lane < kSegTicketBatch) {
                 kind = -1;
                 const unsigned t = base + (unsigned)lane;
-                if (t < p.total_items) seg_decode(t, p, kind, plane, chunk);
+                if (t < p.total_items) seg_tma_decode(t, p, kind, plane, chunk);
                 dec[lane].kind = kind; dec[lane].chunk = chunk; dec[lane].plane = plane;
                 // the lane that decodes a ticket also issues it: the map load overlaps the empty-stage wait below
                 if (kind == 1) splane = src_plane(p.smap, plane);
@@ -688,15 +652,9 @@ __global__ void __launch_bounds__(32 + kSegGroups * kSegGroupThreads + kSegMerge
 #pragma unroll
                         for (int u = 0; u < kUnroll; ++u) {
                             if (c0 + u < hi) {
-                                if (!slot1_valid(v[u])) {
-                                    const float2* sp = base + (int64_t)(c0 + u) * kMaxDense;
-                                    const uint64_t t0 = global_timer_ns();
-                                    do {   // straggling statistics item
-                                        __nanosleep(64);
-                                        v[u] = ld_slot1(sp);
-                                        if (watchdog_expired(t0)) __trap();
-                                    } while (!slot1_valid(v[u]));
-                                }
+                                // a straggling statistics item: wait for it
+                                spin_wait(64, [&] { v[u] = ld_slot1(base + (int64_t)(c0 + u) * kMaxDense); },
+                                          [&] { return slot1_valid(v[u]); });
                                 s4[which * 2 + 0] += (double)v[u].x;
                                 s4[which * 2 + 1] += (double)v[u].y;
                             }
@@ -875,12 +833,9 @@ __global__ void __launch_bounds__(32 + kSegGroups * kSegGroupThreads + kSegMerge
         } else if (kind == 2) {
             // ---------------- apply
             if (plane != cached_apply) {   // group-uniform: wait for the merge item, cache the coefficient table
-                if (lane == 0 && ld_acquire(&p.ready[plane]) == 0) {
-                    const uint64_t t0 = global_timer_ns();
-                    while (ld_acquire(&p.ready[plane]) == 0) {
-                        __nanosleep(64);
-                        if (watchdog_expired(t0)) __trap();
-                    }
+                if (lane == 0) {
+                    int merged = ld_acquire(&p.ready[plane]);
+                    spin_wait(64, [&] { merged = ld_acquire(&p.ready[plane]); }, [&] { return merged != 0; });
                 }
                 named_bar_sync(1 + group, kSegGroupThreads);
                 if (gt < dcount) c_coef[gt] = __ldcg(&p.coef[plane * kLabels + __ldg(p.label_of + sample * kMaxDense + gt)]);
@@ -1025,10 +980,7 @@ int64_t seg_plan_schedule(SegTmaParams& q, bool has_prev) {
     q.imax = q.ic > q.is ? q.ic : q.is;
     q.apply_elems = has_prev ? kSegPrevElems : kSegItemElems;
     q.ia = (int)((q.hw_c + q.apply_elems - 1) / q.apply_elems);
-    const int64_t plane_bytes = q.hw_c * (int64_t)sizeof(float);
-    int64_t lag = (g_knobs.seg_lag_bytes + plane_bytes - 1) / plane_bytes;
-    if (lag < 3) lag = 3;
-    q.lag = (int)(lag < planes ? lag : planes);
+    q.lag = lag_planes(g_knobs.seg_lag_bytes, q.hw_c * (int64_t)sizeof(float), planes);
     return planes * ((int64_t)q.ic + q.is + 1 + q.ia);
 }
 
@@ -1037,7 +989,7 @@ __global__ void seg_schedule_dump_kernel(SegTmaParams p, int32_t* out) {
     if (t >= p.total_items) return;
     int kind = -1, chunk = 0;
     int64_t plane = 0;
-    seg_decode(t, p, kind, plane, chunk);
+    seg_tma_decode(t, p, kind, plane, chunk);
     out[3 * (size_t)t + 0] = kind;
     out[3 * (size_t)t + 1] = (int32_t)plane;
     out[3 * (size_t)t + 2] = chunk;
@@ -1205,11 +1157,8 @@ int seg_adain_fwd_impl(const float* content, const float* style, const uint8_t* 
     const int64_t chunk = (int64_t)kPipeThreads * kPerThread * (vec ? 4 : 1);
     p.ipp_c = (int)((hw_c + chunk - 1) / chunk);
     p.ipp_s = (int)((hw_s + chunk - 1) / chunk);
-    const int64_t plane_bytes = hw_c * (int64_t)sizeof(float);
-    int64_t lag = (g_knobs.adain_lag_bytes + plane_bytes - 1) / plane_bytes;
-    if (lag < 3) lag = 3;
     const int64_t planes = n * c;
-    p.lag = (int)(lag < planes ? lag : planes);
+    p.lag = lag_planes(g_knobs.adain_lag_bytes, hw_c * (int64_t)sizeof(float), planes);
     const int64_t total = planes * (2ll * p.ipp_c + p.ipp_s);
     RPST_CHECK_ARG(total < (1ll << 31), "seg_adain: too many work items (%lld); split the call", (long long)total);
     p.total_items = (unsigned)total;
