@@ -209,6 +209,24 @@ RPST_API int rpst_seg_adain_fwd_mapped(const float* content, const float* style,
                               const int32_t* content_map, const int32_t* style_map, int32_t* label_info,
                               void* workspace, size_t workspace_bytes, void* stream);
 
+/* Backward of rpst_seg_adain_fwd w.r.t. content and style (the reference differentiates its index_select / var /
+ * index_copy_ sequence with autograd; masked training needs the same gradients).  For sample i, channel ch and a
+ * usable label with n_c content pixels, x^ = (c - mu_c)/sd_c, a = sd_s/sd_c, G1 = sum g, G2 = sum g*x^ over those
+ * pixels (g = grad_out):
+ *   content pixel of the label:  dc = a*(g - G1/n_c - x^*G2/(n_c - 1))
+ *   style pixel of the label:    ds = G1/n_s + G2*(s - mu_s)/((n_s - 1)*sd_s)
+ *   content pixel of an unusable label: dc = g bit-exactly; style pixel without a usable label: ds = 0.
+ * d/dprev is grad_out itself.  Shapes and labels as in rpst_seg_adain_fwd (content and style may differ in H*W).
+ * The masked statistics are recomputed here, so no forward state is needed; the result is run-to-run bit-identical.
+ *   grad_content [n,c,hw_c] or NULL, grad_style [n,c,hw_s] or NULL: a NULL half is skipped (style is still read).
+ *   Outputs must not overlap each other or an input.  n*c < 2^31; hw_c, hw_s < 2^31.
+ * Workspace: rpst_seg_adain_bwd_workspace_bytes (from the shapes alone; 256-byte aligned). */
+RPST_API size_t rpst_seg_adain_bwd_workspace_bytes(int64_t n, int64_t c, int64_t hw_c, int64_t hw_s);
+RPST_API int rpst_seg_adain_bwd(const float* grad_out, const float* content, const float* style,
+                       const uint8_t* c_labels, const uint8_t* s_labels, float* grad_content,
+                       float* grad_style, int64_t n, int64_t c, int64_t hw_c, int64_t hw_s, float eps,
+                       void* workspace, size_t workspace_bytes, void* stream);
+
 /* ------------------------------------------------------------------------------------------
  * a12 cal_dist(A, B)                                                  network/base.py:349-360
  *   a [d,m], b [d,n] (d-dimensional column vectors) -> out [m,n] = |a_i|^2 + |b_j|^2 - 2 a_i.b_j

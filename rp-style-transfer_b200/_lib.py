@@ -73,6 +73,8 @@ SIGNATURES = {
     "rpst_seg_adain_fwd": (c_int, [P, P, P, P, P, P, c_int64, c_int64, c_int64, c_int64, c_float, P, P, c_size_t, P]),
     "rpst_seg_adain_fwd_mapped": (c_int, [P, P, P, P, P, P, c_int64, c_int64, c_int64, c_int64, c_int64, c_float,
                                           P, P, P, P, c_size_t, P]),
+    "rpst_seg_adain_bwd_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int64, c_int64]),
+    "rpst_seg_adain_bwd": (c_int, [P, P, P, P, P, P, P, c_int64, c_int64, c_int64, c_int64, c_float, P, c_size_t, P]),
 }
 
 

@@ -13,7 +13,7 @@
 //                     device through a flag, without host synchronisation)
 // The validity rule (network/base.py:435: label taken from the CONTENT map; cnt_c>10, cnt_s>10,
 // cnt_c/cnt_s<100, cnt_s/cnt_c<100) uses exact integer comparisons; pixels of unusable labels are
-// copied through bit-exactly.
+// copied through bit-exactly.  The backward (rpst_seg_adain_bwd) is the seg_bwd_* kernels further down.
 #include "common.cuh"
 #include "tuning.cuh"
 #include "plane_io.cuh"
@@ -967,6 +967,288 @@ int launch_seg_tma(const SegTmaParams& p, cudaStream_t st) {
     return RPST_OK;
 }
 
+// ------------------------------------------------------------------------------------------
+// Backward (rpst_seg_adain_bwd): three stream-ordered phases, no inter-CTA waits.
+//  1. label tables: seg_hist_kernel (counts, first pixels) and seg_shift_kernel (K_l per plane and tensor);
+//  2. seg_bwd_reduce_kernel, one CTA per (plane, chunk): per-label shifted sums of the chunk, written as one partial
+//     row per usable label -- content chunks (S1, S2, G1, G2) = sum (c-K), (c-K)^2, g, g*(c-K); style chunks (S1, S2);
+//  3. seg_bwd_coef_kernel merges a plane's rows in chunk order in fp64 into dc = a*g + b + y*(c - mu_c) and
+//     ds = d + e*(s - mu_s); seg_bwd_apply_kernel streams g, c, s and the labels to write dc and ds.
+// Every sum is taken in a fixed order (lane runs, lane-ordered groups per label, warps in index order, chunks in
+// index order), so the gradients are run-to-run bit-identical for every label map.
+// ------------------------------------------------------------------------------------------
+constexpr int kBwdWarps = 8;
+constexpr int kBwdThreads = kBwdWarps * 32;
+constexpr int kBwdLanePixels = 16;                                  // contiguous pixels of one lane per tile
+constexpr int kBwdTilePixels = 32 * kBwdLanePixels;                 // one warp
+constexpr int kBwdChunk = 65536;                                    // pixels of one reduce / apply CTA
+constexpr int kBwdTiles = kBwdChunk / (kBwdWarps * kBwdTilePixels); // tiles per warp
+static_assert(kBwdThreads == kLabels, "one thread per label value in the merge of the warp tables");
+
+struct SegBwdParams {
+    const float* g;
+    const float* content;
+    const float* style;
+    const uint8_t* c_lab;
+    const uint8_t* s_lab;
+    float* dc;                // may be null
+    float* ds;                // may be null
+    int64_t channels, hw_c, hw_s;
+    float eps;
+    int ic, is;               // content / style chunks per plane
+    const int* cnt;           // [n][2][256]
+    const float* shift;       // [planes][2][256]
+    float4* part;             // [planes][ic + is][256]: content rows (S1, S2, G1, G2), style rows (S1, S2, 0, 0)
+    float4* coef;             // [planes][2][256]: content (a, b, y, mu_c), style (d, e, mu_s, 0)
+};
+
+// One flush of open label runs into the warp's table: lanes holding the same label form a group (match.any) whose
+// lowest lane adds the others' sums in lane order, then adds the group total to tab[key].  key < 0: nothing to flush.
+template <int NS>
+__device__ __forceinline__ void bwd_warp_flush(float4* tab, int lane, int key, const float (&a)[4]) {
+    const unsigned peers = __match_any_sync(0xffffffffu, key);
+    const int steps = (int)__reduce_max_sync(0xffffffffu, (unsigned)__popc(peers));
+    float s[4] = {a[0], a[1], a[2], a[3]};
+    unsigned rem = peers & (peers - 1u);
+    for (int k = 1; k < steps; ++k) {
+        const int src = rem ? __ffs(rem) - 1 : lane;
+#pragma unroll
+        for (int q = 0; q < NS; ++q) {
+            const float x = __shfl_sync(0xffffffffu, a[q], src);
+            if (rem) s[q] += x;
+        }
+        rem &= rem - 1u;
+    }
+    if (key >= 0 && (peers & ((1u << lane) - 1u)) == 0u) {
+        float4 t = tab[key];
+        t.x += s[0]; t.y += s[1];
+        if (NS == 4) { t.z += s[2]; t.w += s[3]; }
+        tab[key] = t;
+    }
+    __syncwarp();
+}
+
+template <int VEC>
+__device__ __forceinline__ void load_px(float (&v)[VEC], const float* p) {
+    if constexpr (VEC == 4) {
+        const float4 q = __ldg(reinterpret_cast<const float4*>(p));
+        v[0] = q.x; v[1] = q.y; v[2] = q.z; v[3] = q.w;
+    } else {
+        v[0] = __ldg(p);
+    }
+}
+
+// Per-label sums of one chunk into the warp tables.  CONTENT: (S1, S2, G1, G2), else (S1, S2).  Each lane owns
+// kBwdLanePixels contiguous pixels per tile, so label runs stay whole on blocky maps; a run is carried across the
+// lane's pixels until its label changes, and changes are flushed by the whole warp.
+template <int VEC, bool CONTENT>
+__device__ __forceinline__ void bwd_reduce_chunk(float4* tab, const float* x, const float* g, const uint8_t* lab,
+                                                 int64_t e0, int64_t hw, const float* s_shift,
+                                                 const unsigned char* s_use) {
+    constexpr int NS = CONTENT ? 4 : 2;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    int cur = -1;
+    float shift = 0.f;
+    float a[4] = {0.f, 0.f, 0.f, 0.f};
+    for (int t = 0; t < kBwdTiles; ++t) {
+        const int64_t w0 = e0 + (int64_t)(t * kBwdWarps + warp) * kBwdTilePixels;
+        if (w0 >= hw) break;   // warp-uniform
+        const int64_t p0 = w0 + lane * kBwdLanePixels;
+#pragma unroll
+        for (int j = 0; j < kBwdLanePixels / VEC; ++j) {
+            const int64_t p = p0 + j * VEC;
+            const bool in = p < hw;   // VEC == 4 needs hw % 4 == 0: a vector is wholly in or out
+            float xv[VEC], gv[VEC];
+            int lv[VEC];
+            if (in) {
+                load_px<VEC>(xv, x + p);
+                if (CONTENT) load_px<VEC>(gv, g + p);
+                load_labels<VEC>(lv, lab + p);
+            }
+            // fast path: the whole warp continues its runs over these VEC pixels
+            bool same = in && cur >= 0;
+#pragma unroll
+            for (int e = 0; e < VEC; ++e) same = same && lv[e] == cur;
+            if (VEC > 1 && __all_sync(0xffffffffu, same)) {
+#pragma unroll
+                for (int e = 0; e < VEC; ++e) {
+                    const float d = xv[e] - shift;
+                    a[0] += d;
+                    a[1] = fmaf(d, d, a[1]);
+                    if (CONTENT) { a[2] += gv[e]; a[3] = fmaf(gv[e], d, a[3]); }
+                }
+                continue;
+            }
+#pragma unroll
+            for (int e = 0; e < VEC; ++e) {
+                const int key = in && s_use[lv[e]] ? lv[e] : -1;
+                const bool brk = key != cur;
+                if (__any_sync(0xffffffffu, brk && cur >= 0)) bwd_warp_flush<NS>(tab, lane, brk ? cur : -1, a);
+                if (brk) {
+                    cur = key;
+                    shift = key >= 0 ? s_shift[key] : 0.f;
+                    a[0] = a[1] = a[2] = a[3] = 0.f;
+                }
+                if (cur >= 0) {
+                    const float d = xv[e] - shift;
+                    a[0] += d;
+                    a[1] = fmaf(d, d, a[1]);
+                    if (CONTENT) { a[2] += gv[e]; a[3] = fmaf(gv[e], d, a[3]); }
+                }
+            }
+        }
+    }
+    bwd_warp_flush<NS>(tab, lane, cur, a);
+}
+
+template <int VEC>
+__global__ void __launch_bounds__(kBwdThreads) seg_bwd_reduce_kernel(SegBwdParams p) {
+    __shared__ float4 s_tab[kBwdWarps][kLabels];
+    __shared__ float s_shift[kLabels];
+    __shared__ unsigned char s_use[kLabels];
+    const int items = p.ic + p.is;
+    const int64_t plane = blockIdx.x / items;
+    const int chunk = (int)(blockIdx.x % items);
+    const int64_t sample = plane / p.channels;
+    const bool is_style = chunk >= p.ic;
+    const int l = threadIdx.x;
+    const bool use = label_usable(__ldg(p.cnt + sample * 2 * kLabels + l), __ldg(p.cnt + (sample * 2 + 1) * kLabels + l));
+    s_use[l] = use;
+    s_shift[l] = __ldg(p.shift + (plane * 2 + is_style) * kLabels + l);
+#pragma unroll
+    for (int w = 0; w < kBwdWarps; ++w) s_tab[w][l] = make_float4(0.f, 0.f, 0.f, 0.f);
+    __syncthreads();
+    float4* tab = s_tab[threadIdx.x >> 5];
+    if (is_style) {
+        bwd_reduce_chunk<VEC, false>(tab, p.style + plane * p.hw_s, nullptr, p.s_lab + sample * p.hw_s,
+                                     (int64_t)(chunk - p.ic) * kBwdChunk, p.hw_s, s_shift, s_use);
+    } else {
+        bwd_reduce_chunk<VEC, true>(tab, p.content + plane * p.hw_c, p.g + plane * p.hw_c, p.c_lab + sample * p.hw_c,
+                                    (int64_t)chunk * kBwdChunk, p.hw_c, s_shift, s_use);
+    }
+    __syncthreads();
+    if (use) {
+        float4 r = s_tab[0][l];
+#pragma unroll
+        for (int w = 1; w < kBwdWarps; ++w) {
+            const float4 q = s_tab[w][l];
+            r.x += q.x; r.y += q.y; r.z += q.z; r.w += q.w;
+        }
+        p.part[(plane * items + chunk) * kLabels + l] = r;
+    }
+}
+
+// One thread per (plane, label): the plane's partial rows in chunk order, in fp64, into the gradient coefficients.
+__global__ void __launch_bounds__(kLabels) seg_bwd_coef_kernel(SegBwdParams p) {
+    const int64_t plane = blockIdx.x, sample = plane / p.channels;
+    const int l = threadIdx.x;
+    const int nci = __ldg(p.cnt + sample * 2 * kLabels + l), nsi = __ldg(p.cnt + (sample * 2 + 1) * kLabels + l);
+    if (!label_usable(nci, nsi)) return;   // the apply kernel copies g / writes 0 for these labels
+    const int items = p.ic + p.is;
+    const float4* row = p.part + plane * items * kLabels + l;
+    double s1c = 0.0, s2c = 0.0, g1 = 0.0, g2 = 0.0, s1s = 0.0, s2s = 0.0;
+#pragma unroll 8
+    for (int k = 0; k < p.ic; ++k) {
+        const float4 v = row[(int64_t)k * kLabels];
+        s1c += v.x; s2c += v.y; g1 += v.z; g2 += v.w;
+    }
+#pragma unroll 8
+    for (int k = p.ic; k < items; ++k) {
+        const float4 v = row[(int64_t)k * kLabels];
+        s1s += v.x; s2s += v.y;
+    }
+    const double nc = nci, ns = nsi, eps = p.eps;
+    const double dmc = s1c / nc, dms = s1s / ns;   // mu - K
+    const double sd_c = sqrt(fmax(s2c - s1c * dmc, 0.0) / (nc - 1.0) + eps);
+    const double sd_s = sqrt(fmax(s2s - s1s * dms, 0.0) / (ns - 1.0) + eps);
+    const double gx = (g2 - g1 * dmc) / sd_c;      // G2 = sum g * (c - mu_c) / sd_c
+    const double a = sd_s / sd_c;
+    const double kc = __ldg(p.shift + plane * 2 * kLabels + l), ks = __ldg(p.shift + (plane * 2 + 1) * kLabels + l);
+    p.coef[(plane * 2 + 0) * kLabels + l] =
+        make_float4((float)a, (float)(-a * g1 / nc), (float)(-a * gx / ((nc - 1.0) * sd_c)), (float)(kc + dmc));
+    p.coef[(plane * 2 + 1) * kLabels + l] =
+        make_float4((float)(g1 / ns), (float)(gx / ((ns - 1.0) * sd_s)), (float)(ks + dms), 0.f);
+}
+
+// dc = a*g + b + y*(c - mu_c) on usable labels, g itself elsewhere; ds = d + e*(s - mu_s) on usable labels, 0 elsewhere.
+template <int VEC>
+__global__ void __launch_bounds__(kBwdThreads) seg_bwd_apply_kernel(SegBwdParams p) {
+    __shared__ float4 s_coef[kLabels];
+    __shared__ unsigned char s_use[kLabels];
+    const int ac = p.dc ? p.ic : 0, as = p.ds ? p.is : 0, items = ac + as;
+    const int64_t plane = blockIdx.x / items;
+    const int chunk = (int)(blockIdx.x % items);
+    const int64_t sample = plane / p.channels;
+    const bool is_style = chunk >= ac;
+    const int l = threadIdx.x;
+    s_use[l] = label_usable(__ldg(p.cnt + sample * 2 * kLabels + l), __ldg(p.cnt + (sample * 2 + 1) * kLabels + l));
+    s_coef[l] = p.coef[(plane * 2 + is_style) * kLabels + l];   // unusable labels: stale values, never read
+    __syncthreads();
+    const int64_t hw = is_style ? p.hw_s : p.hw_c;
+    const int64_t e0 = (int64_t)(is_style ? chunk - ac : chunk) * kBwdChunk;
+    const int64_t e1 = e0 + kBwdChunk < hw ? e0 + kBwdChunk : hw;
+    const uint8_t* lab = is_style ? p.s_lab + sample * hw : p.c_lab + sample * hw;
+    if (is_style) {
+        const float* s = p.style + plane * hw;
+        float* out = p.ds + plane * hw;
+        for (int64_t i = e0 + (int64_t)threadIdx.x * VEC; i < e1; i += kBwdThreads * VEC) {
+            float v[VEC], o[VEC];
+            int lv[VEC];
+            load_px<VEC>(v, s + i);
+            load_labels<VEC>(lv, lab + i);
+#pragma unroll
+            for (int e = 0; e < VEC; ++e) {
+                if (s_use[lv[e]]) {
+                    const float4 cf = s_coef[lv[e]];
+                    o[e] = fmaf(cf.y, v[e] - cf.z, cf.x);
+                } else {
+                    o[e] = 0.f;
+                }
+            }
+            store_vec<VEC>(out + i, o, 0, false);
+        }
+    } else {
+        const float* c = p.content + plane * hw;
+        const float* g = p.g + plane * hw;
+        float* out = p.dc + plane * hw;
+        for (int64_t i = e0 + (int64_t)threadIdx.x * VEC; i < e1; i += kBwdThreads * VEC) {
+            float v[VEC], gv[VEC], o[VEC];
+            int lv[VEC];
+            load_px<VEC>(v, c + i);
+            load_px<VEC>(gv, g + i);
+            load_labels<VEC>(lv, lab + i);
+#pragma unroll
+            for (int e = 0; e < VEC; ++e) {
+                if (s_use[lv[e]]) {
+                    const float4 cf = s_coef[lv[e]];
+                    o[e] = fmaf(cf.z, v[e] - cf.w, fmaf(cf.x, gv[e], cf.y));
+                } else {
+                    o[e] = gv[e];   // the forward copies these pixels through
+                }
+            }
+            store_vec<VEC>(out + i, o, 0, false);
+        }
+    }
+}
+
+struct SegBwdLayout {
+    size_t cnt, first, shift, coef, part, total;
+};
+SegBwdLayout seg_bwd_layout(int64_t n, int64_t c, int64_t hw_c, int64_t hw_s) {
+    const size_t planes = (size_t)(n * c);
+    const size_t items = (size_t)((hw_c + kBwdChunk - 1) / kBwdChunk + (hw_s + kBwdChunk - 1) / kBwdChunk);
+    SegBwdLayout l;
+    size_t o = 0;
+    auto take = [&](size_t bytes) { size_t at = o; o += align_up(bytes, 256); return at; };
+    l.cnt = take((size_t)n * 2 * kLabels * sizeof(int));
+    l.first = take((size_t)n * 2 * kLabels * sizeof(int));
+    l.shift = take(planes * 2 * kLabels * sizeof(float));
+    l.coef = take(planes * 2 * kLabels * sizeof(float4));
+    l.part = take(planes * items * kLabels * sizeof(float4));
+    l.total = o;
+    return l;
+}
+
 }  // namespace
 }  // namespace rpst
 
@@ -1170,5 +1452,90 @@ int seg_adain_fwd_impl(const float* content, const float* style, const uint8_t* 
     return RPST_OK;
 }
 }  // namespace
+
+extern "C" size_t rpst_seg_adain_bwd_workspace_bytes(int64_t n, int64_t c, int64_t hw_c, int64_t hw_s) {
+    if (n <= 0 || c <= 0 || hw_c <= 0 || hw_s <= 0) return 256;
+    return seg_bwd_layout(n, c, hw_c, hw_s).total;
+}
+
+namespace {
+bool overlaps(const void* a, int64_t a_bytes, const void* b, int64_t b_bytes) {
+    if (a == nullptr || b == nullptr) return false;
+    const uintptr_t x = reinterpret_cast<uintptr_t>(a), y = reinterpret_cast<uintptr_t>(b);
+    return x < y + (uint64_t)b_bytes && y < x + (uint64_t)a_bytes;
+}
+}  // namespace
+
+extern "C" int rpst_seg_adain_bwd(const float* grad_out, const float* content, const float* style,
+                                  const uint8_t* c_labels, const uint8_t* s_labels, float* grad_content,
+                                  float* grad_style, int64_t n, int64_t c, int64_t hw_c, int64_t hw_s, float eps,
+                                  void* workspace, size_t workspace_bytes, void* stream) {
+    RPST_CHECK_ARG(n >= 0 && c >= 0 && hw_c >= 0 && hw_s >= 0, "seg_adain_bwd: negative size");
+    if (n == 0 || c == 0) return RPST_OK;
+    RPST_CHECK_ARG(grad_out && content && style && c_labels && s_labels, "seg_adain_bwd: null pointer");
+    RPST_CHECK_ARG(hw_c > 0 && hw_s > 0, "seg_adain_bwd: empty plane");
+    RPST_CHECK_ARG(n * c < (1ll << 31), "seg_adain_bwd: plane index does not fit int32");
+    RPST_CHECK_ARG(hw_c < (1ll << 31) && hw_s < (1ll << 31), "seg_adain_bwd: plane too large");
+    const int64_t planes = n * c;
+    const int64_t ic = (hw_c + kBwdChunk - 1) / kBwdChunk, is = (hw_s + kBwdChunk - 1) / kBwdChunk;
+    RPST_CHECK_ARG(planes * (ic + is) < (1ll << 31), "seg_adain_bwd: too many work items (%lld); split the call",
+                   (long long)(planes * (ic + is)));
+    const int64_t bc = planes * hw_c * 4, bs = planes * hw_s * 4;
+    const void* inputs[5] = {grad_out, content, style, c_labels, s_labels};
+    const int64_t in_bytes[5] = {bc, bc, bs, n * hw_c, n * hw_s};
+    for (int i = 0; i < 5; ++i) {
+        RPST_CHECK_ARG(!overlaps(grad_content, bc, inputs[i], in_bytes[i]) && !overlaps(grad_style, bs, inputs[i], in_bytes[i]),
+                       "seg_adain_bwd: grad_content / grad_style must not alias an input");
+    }
+    RPST_CHECK_ARG(!overlaps(grad_content, bc, grad_style, bs), "seg_adain_bwd: grad_content and grad_style overlap");
+    const size_t need = rpst_seg_adain_bwd_workspace_bytes(n, c, hw_c, hw_s);
+    if (workspace == nullptr || workspace_bytes < need) {
+        set_error("seg_adain_bwd: workspace too small (%zu < %zu bytes)", workspace_bytes, need);
+        return RPST_ERR_WORKSPACE;
+    }
+    RPST_CHECK_ARG(aligned(workspace, 256), "seg_adain_bwd: workspace must be 256-byte aligned");
+    if (grad_content == nullptr && grad_style == nullptr) return RPST_OK;
+
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    char* base = static_cast<char*>(workspace);
+    const SegBwdLayout w = seg_bwd_layout(n, c, hw_c, hw_s);
+    int* cnt = reinterpret_cast<int*>(base + w.cnt);
+    int* first = reinterpret_cast<int*>(base + w.first);
+    float* shift = reinterpret_cast<float*>(base + w.shift);
+    RPST_CUDA(cudaMemsetAsync(cnt, 0, w.first - w.cnt, st));
+    RPST_CUDA(cudaMemsetAsync(first, 0x7f, w.shift - w.first, st));
+    const int64_t hw_max = hw_c > hw_s ? hw_c : hw_s;
+    int hist_blocks = (int)((hw_max + 16383) / 16384);
+    if (hist_blocks > 256) hist_blocks = 256;
+    seg_hist_kernel<<<dim3(hist_blocks, (unsigned)n, 2), 256, 0, st>>>(c_labels, s_labels, hw_c, hw_s, cnt, first);
+    RPST_CUDA(cudaGetLastError());
+    SegTmaParams q{};
+    q.content = content; q.style = style; q.n = n; q.channels = c; q.hw_c = hw_c; q.hw_s = hw_s;
+    q.cnt = cnt; q.first = first; q.shift = shift;
+    seg_shift_kernel<<<(unsigned)((planes * 2 * kLabels + 255) / 256), 256, 0, st>>>(q);
+    RPST_CUDA(cudaGetLastError());
+
+    SegBwdParams p{};
+    p.g = grad_out; p.content = content; p.style = style; p.c_lab = c_labels; p.s_lab = s_labels;
+    p.dc = grad_content; p.ds = grad_style;
+    p.channels = c; p.hw_c = hw_c; p.hw_s = hw_s; p.eps = eps; p.ic = (int)ic; p.is = (int)is;
+    p.cnt = cnt; p.shift = shift;
+    p.part = reinterpret_cast<float4*>(base + w.part);
+    p.coef = reinterpret_cast<float4*>(base + w.coef);
+    const bool vec = hw_c % 4 == 0 && hw_s % 4 == 0 && aligned(grad_out, 16) && aligned(content, 16) &&
+                     aligned(style, 16) && (!grad_content || aligned(grad_content, 16)) &&
+                     (!grad_style || aligned(grad_style, 16)) && aligned(c_labels, 4) && aligned(s_labels, 4);
+    const unsigned reduce_grid = (unsigned)(planes * (ic + is));
+    if (vec) seg_bwd_reduce_kernel<4><<<reduce_grid, kBwdThreads, 0, st>>>(p);
+    else seg_bwd_reduce_kernel<1><<<reduce_grid, kBwdThreads, 0, st>>>(p);
+    RPST_CUDA(cudaGetLastError());
+    seg_bwd_coef_kernel<<<(unsigned)planes, kLabels, 0, st>>>(p);
+    RPST_CUDA(cudaGetLastError());
+    const unsigned apply_grid = (unsigned)(planes * ((grad_content ? ic : 0) + (grad_style ? is : 0)));
+    if (vec) seg_bwd_apply_kernel<4><<<apply_grid, kBwdThreads, 0, st>>>(p);
+    else seg_bwd_apply_kernel<1><<<apply_grid, kBwdThreads, 0, st>>>(p);
+    RPST_CUDA(cudaGetLastError());
+    return RPST_OK;
+}
 
 RPST_WATCHDOG_SETTER(seg)

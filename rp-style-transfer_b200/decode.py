@@ -5,6 +5,7 @@ The reference spells the multiscale blend as two ops, `stylized + AdaIN(c_l, s_l
 installed over `<Class>.decode` by `rpst.install()` and also usable directly (`multiscale_transform`)."""
 from __future__ import annotations
 
+import functools
 from typing import List, Sequence
 
 import torch
@@ -25,13 +26,14 @@ def multiscale_transform(content_feats: Sequence[torch.Tensor], style_feats: Seq
 
 
 def decode_multiscale(self, content_feats, style_feats, use_mask=False, c_mask_path=None, s_mask_path=None,
-                      plane_maps=None):
+                      plane_maps=None, *, segment_grad=False):
     """MultiScaleAdaINRPNet.decode (network/adain_rp.py:286-302): top level plain (seg-)AdaIN, every
     shallower level `decoder(prev + (seg-)AdaIN(c_l, s_l))` with the add fused into the transform.
     `sort_by_weights` (:230-249, applied here when `self._sort`) and the channel `shuffle` of `test()`
     (:256-260, handed over as `plane_maps` by `test_multiscale`) become plane maps of the kernel call
     instead of permuted copies, in the masked (segment AdaIN) branch too.  Like the reference, content and
-    style are sorted by the SAME attention weights (the ones the shared encoder stored last)."""
+    style are sorted by the SAME attention weights (the ones the shared encoder stored last).  `segment_grad`
+    records the masked levels for autograd (`differentiable=True` of segment AdaIN)."""
     levels = len(content_feats)
     maps = list(plane_maps) if plane_maps is not None else [None] * levels
     if self._sort:
@@ -42,7 +44,7 @@ def decode_multiscale(self, content_feats, style_feats, use_mask=False, c_mask_p
         cf, sf = content_feats[l], style_feats[l]
         if use_mask:
             return SEG.do_mask_stylized(cf, sf, c_mask_path, s_mask_path, prev=prev, content_map=maps[l],
-                                        style_map=maps[l])
+                                        style_map=maps[l], differentiable=segment_grad)
         if maps[l] is not None:
             return F.adain_mapped(cf, sf, maps[l], maps[l], prev=prev)
         return F.adaptive_instance_normalization(cf, sf) if prev is None else F.adain_blend(prev, cf, sf)
@@ -60,7 +62,8 @@ def test_multiscale(self, content, style, iterations=0, bid=0, c_mask_path=None,
     with torch.no_grad():
         content_feats = self.encode_rp_intermediate(content)
         style_feats = self.encode_rp_intermediate(style)
-        if getattr(type(self), "decode", decode_multiscale) is decode_multiscale:
+        decode = getattr(type(self), "decode", decode_multiscale)
+        if getattr(decode, "__wrapped__", decode) is decode_multiscale:
             maps = None
             if self._shuffle:
                 maps = [None if idx > self._shuffle_layers else
@@ -79,22 +82,26 @@ def test_multiscale(self, content, style, iterations=0, bid=0, c_mask_path=None,
         return stylized
 
 
-def _top(self, content_feats, style_feats, use_mask, c_mask_path, s_mask_path):
+def _top(self, content_feats, style_feats, use_mask, c_mask_path, s_mask_path, segment_grad):
     if use_mask:
-        return SEG.do_mask_stylized(content_feats[-1], style_feats[-1], c_mask_path, s_mask_path)
+        return SEG.do_mask_stylized(content_feats[-1], style_feats[-1], c_mask_path, s_mask_path,
+                                    differentiable=segment_grad)
     return F.adaptive_instance_normalization(content_feats[-1], style_feats[-1])
 
 
-def decode_ldms(self, content_feats, style_feats, use_mask=False, c_mask_path=None, s_mask_path=None):
+def decode_ldms(self, content_feats, style_feats, use_mask=False, c_mask_path=None, s_mask_path=None, *,
+                segment_grad=False):
     """LDMSAdaINRPNet.decode (network/adain_rp.py:538-553; inherited by LDMS 2/3): decoder blocks are
     attributes `rp_dec{i}`; lower levels use the running decoder state as content,
-    `stylized + AdaIN(stylized, s_l)` (prev aliases content), only while `i < stylized_layers-1`."""
-    stylized = self.rp_dec0(_top(self, content_feats, style_feats, use_mask, c_mask_path, s_mask_path))
+    `stylized + AdaIN(stylized, s_l)` (prev aliases content), only while `i < stylized_layers-1`.
+    `segment_grad` as in `decode_multiscale`."""
+    stylized = self.rp_dec0(_top(self, content_feats, style_feats, use_mask, c_mask_path, s_mask_path, segment_grad))
     lower = list(zip(content_feats[:-1], style_feats[:-1]))[::-1]
     for i, (cf, sf) in enumerate(lower):
         if i < self.stylized_layers - 1:
             if use_mask:
-                fused = SEG.do_mask_stylized(cf, sf, c_mask_path, s_mask_path, prev=stylized)
+                fused = SEG.do_mask_stylized(cf, sf, c_mask_path, s_mask_path, prev=stylized,
+                                             differentiable=segment_grad)
             else:
                 fused = F.adain_blend(stylized, stylized, sf)
         else:
@@ -103,17 +110,19 @@ def decode_ldms(self, content_feats, style_feats, use_mask=False, c_mask_path=No
     return stylized
 
 
-def decode_ld_concat(self, content_feats, style_feats, use_mask=False, c_mask_path=None, s_mask_path=None):
+def decode_ld_concat(self, content_feats, style_feats, use_mask=False, c_mask_path=None, s_mask_path=None, *,
+                     segment_grad=False):
     """LDMSAdaINRPNet4.decode (network/adain_rp.py:780-799, inherited by LDMS 5):
-    `cat([stylized, (seg-)AdaIN(c_l, s_l)], 1)` with the AdaIN half written straight into the result."""
-    stylized = self.rp_dec0(_top(self, content_feats, style_feats, use_mask, c_mask_path, s_mask_path))
+    `cat([stylized, (seg-)AdaIN(c_l, s_l)], 1)` with the AdaIN half written straight into the result.
+    `segment_grad` as in `decode_multiscale`."""
+    stylized = self.rp_dec0(_top(self, content_feats, style_feats, use_mask, c_mask_path, s_mask_path, segment_grad))
     lower = list(zip(content_feats[:-1], style_feats[:-1]))[::-1]
     for i, (cf, sf) in enumerate(lower):
         if use_mask:
             hc, wc = cf.shape[2:]
             hs, ws = sf.shape[2:]
             fused = SEG.seg_adain_concat(stylized, cf, sf, SEG.stack_label_maps(c_mask_path, wc, hc, cf.device),
-                                         SEG.stack_label_maps(s_mask_path, ws, hs, sf.device))
+                                         SEG.stack_label_maps(s_mask_path, ws, hs, sf.device), differentiable=segment_grad)
         else:
             fused = F.adain_concat(stylized, cf, sf)
         stylized = getattr(self, f'rp_dec{i + 1}')(fused)
@@ -127,3 +136,14 @@ PATCHED_DECODES = {
     "LDMSAdaINRPNet": decode_ldms,
     "LDMSAdaINRPNet4": decode_ld_concat,
 }
+
+
+def _with_segment_grad(decode):
+    @functools.wraps(decode)
+    def wrapper(self, *args, **kwargs):
+        return decode(self, *args, segment_grad=True, **kwargs)
+    return wrapper
+
+
+# the decodes `install(segment_grad=True)` binds: masked levels differentiable, so masked training loops run
+SEGMENT_GRAD_DECODES = {name: _with_segment_grad(fn) for name, fn in PATCHED_DECODES.items()}

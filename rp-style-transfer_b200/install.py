@@ -7,6 +7,7 @@ star-imports network.base everywhere, so each namespace is patched, not just `ne
 (SURVEY.md §7).  `uninstall()` restores the originals."""
 from __future__ import annotations
 
+import functools
 import sys
 from typing import Dict, List, Tuple
 
@@ -17,7 +18,7 @@ from . import mrf as MRF
 from . import sanet as SA
 from . import segment as SEG
 from . import wct as WCT
-from .decode import PATCHED_DECODES, PATCHED_TESTS
+from .decode import PATCHED_DECODES, PATCHED_TESTS, SEGMENT_GRAD_DECODES
 
 # reference name -> replacement (applied wherever the name exists in a network.* namespace)
 NAME_MAP = {
@@ -50,16 +51,24 @@ def _patch(obj, name, value):
     setattr(obj, name, value)
 
 
-def install(package: str = "network") -> Dict[str, int]:
-    """Patch every imported `<package>.*` module; returns {name: number of namespaces patched}."""
+def install(package: str = "network", segment_grad: bool = False) -> Dict[str, int]:
+    """Patch every imported `<package>.*` module; returns {name: number of namespaces patched}.
+    `segment_grad=True` makes segment AdaIN differentiable wherever it is patched in (`AdaINSeg`,
+    `do_mask_stylized` and the masked branches of the decodes), so masked training loops run under autograd."""
     if _saved:
         return {}
     counts: Dict[str, int] = {}
+    name_map = NAME_MAP
+    decodes = PATCHED_DECODES
+    if segment_grad:
+        seg = functools.partial(SEG.adaptive_instance_normalization_with_segment, differentiable=True)
+        name_map = dict(NAME_MAP, adaptive_instance_normalization_with_segment=seg, AdaINSeg=seg)
+        decodes = SEGMENT_GRAD_DECODES
     mods = [m for n, m in list(sys.modules.items()) if m is not None and (n == package or n.startswith(package + "."))]
     if not mods:
         raise RuntimeError(f"rpst.install: package '{package}' is not imported")
     for mod in mods:
-        for name, repl in NAME_MAP.items():
+        for name, repl in name_map.items():
             if name in vars(mod) and vars(mod)[name] is not repl:
                 _patch(mod, name, repl)
                 counts[name] = counts.get(name, 0) + 1
@@ -77,8 +86,8 @@ def install(package: str = "network") -> Dict[str, int]:
                 if "whiten_and_color" in vars(cls):
                     _patch(cls, "whiten_and_color", lambda self, cF, sF, method="closed-form": WCT.whiten_and_color(cF, sF, method))
                     counts["WCTRPNet.whiten_and_color"] = counts.get("WCTRPNet.whiten_and_color", 0) + 1
-            if cname in PATCHED_DECODES and "decode" in vars(cls):
-                _patch(cls, "decode", PATCHED_DECODES[cname])
+            if cname in decodes and "decode" in vars(cls):
+                _patch(cls, "decode", decodes[cname])
                 counts[cname + ".decode"] = 1
             if cname in PATCHED_TESTS and "test" in vars(cls):
                 _patch(cls, "test", PATCHED_TESTS[cname])
@@ -92,7 +101,8 @@ def install(package: str = "network") -> Dict[str, int]:
                        lambda self, input, target, norm=False: LOSS.calc_content_loss(input, target, norm))
                 counts["calc_content_loss"] = counts.get("calc_content_loss", 0) + 1
             if "do_mask_stylized" in vars(cls):
-                _patch(cls, "do_mask_stylized", lambda self, cf, sf, cm, sm: SEG.do_mask_stylized(cf, sf, cm, sm))
+                _patch(cls, "do_mask_stylized",
+                       lambda self, cf, sf, cm, sm: SEG.do_mask_stylized(cf, sf, cm, sm, differentiable=segment_grad))
                 counts["do_mask_stylized"] = counts.get("do_mask_stylized", 0) + 1
     return counts
 

@@ -46,11 +46,16 @@ def stack_label_maps(masks: Union[torch.Tensor, Sequence[LabelArg]], width: int,
     return torch.stack([load_label_map(m, width, height, device) for m in masks], dim=0)
 
 
+def _needs_grad(*tensors) -> bool:
+    return torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in tensors)
+
+
 def _refuse_grad(*tensors) -> None:
-    if torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in tensors):
+    if _needs_grad(*tensors):
         raise NotImplementedError(
             "rpst: segment AdaIN has no backward pass (the reference only calls it from test() under "
-            "torch.no_grad(), network/adain_rp.py:251-262); call it under torch.no_grad() or detach the inputs")
+            "torch.no_grad(), network/adain_rp.py:251-262); call it under torch.no_grad() or detach the inputs.  "
+            "Pass differentiable=True to get gradients for content, style and prev.")
 
 
 def _seg_adain_into(out, out_batch_stride, content_feat, style_feat, c_labels, s_labels, prev, content_map, style_map,
@@ -77,18 +82,78 @@ def _seg_adain_into(out, out_batch_stride, content_feat, style_feat, c_labels, s
     return info
 
 
+class _SegAdaINFn(torch.autograd.Function):
+    """(out [+ prev], label table) of segment AdaIN; the backward recomputes the masked statistics in
+    rpst_seg_adain_bwd, so the forward saves only its inputs (and nothing when only `prev` needs grad)."""
+
+    @staticmethod
+    def forward(ctx, content, style, c_labels, s_labels, prev, want_info):
+        out = torch.empty_like(content)
+        n, ch, hc, wc = content.shape
+        info = _seg_adain_into(out, ch * hc * wc, content, style, c_labels, s_labels, prev, None, None, want_info)
+        if content.requires_grad or style.requires_grad:
+            ctx.save_for_backward(content, style, c_labels, s_labels)
+        ctx.has_prev = prev is not None
+        if info is None:
+            return out
+        ctx.mark_non_differentiable(info)
+        return out, info
+
+    @staticmethod
+    def backward(ctx, grad_out, *_):
+        need_c, need_s, _, _, need_p, _ = ctx.needs_input_grad
+        dc = ds = None
+        if need_c or need_s:
+            content, style, cl, sl = ctx.saved_tensors
+            g = grad_out.contiguous()
+            n, ch, hc, wc = content.shape
+            hs, ws_ = style.shape[2:]
+            dc = torch.empty_like(content) if need_c else None
+            ds = torch.empty_like(style) if need_s else None
+            L = _lib.lib()
+            ws = _workspace(L.rpst_seg_adain_bwd_workspace_bytes(n, ch, hc * wc, hs * ws_), content.device)
+            _lib.check(L.rpst_seg_adain_bwd(g.data_ptr(), content.data_ptr(), style.data_ptr(), cl.data_ptr(),
+                                            sl.data_ptr(), _ptr(dc), _ptr(ds), n, ch, hc * wc, hs * ws_, EPS,
+                                            ws.data_ptr(), ws.numel(), _stream()))
+        return dc, ds, None, None, (grad_out if ctx.has_prev and need_p else None), None
+
+
+def _seg_adain_grad(content_feat, style_feat, c_labels, s_labels, prev, content_map, style_map, want_info):
+    """Differentiable segment AdaIN: plane maps are gathered through autograd (as `adain_mapped` does), then the
+    unmapped kernel pair runs."""
+    c = _prep(content_feat, "content_feat")
+    s = _prep(style_feat, "style_feat")
+    n, ch = c.shape[:2]
+    cm, sm = _check_map(content_map, "content_map", n * ch), _check_map(style_map, "style_map", n * ch)
+    cg = c if cm is None else c.flatten(0, 1)[cm.long()].view_as(c)
+    sg = s if sm is None else s.flatten(0, 1)[sm.long()].view_as(s)
+    p = None if prev is None else _prep(prev, "prev")
+    assert c_labels.dtype == torch.uint8 and s_labels.dtype == torch.uint8 and c_labels.is_cuda and s_labels.is_cuda
+    assert tuple(c_labels.shape) == (n,) + tuple(c.shape[2:]) and tuple(s_labels.shape) == (n,) + tuple(s.shape[2:])
+    if p is not None:
+        assert p.shape == c.shape
+    return _SegAdaINFn.apply(cg.contiguous(), sg.contiguous(), c_labels.contiguous(), s_labels.contiguous(), p,
+                             want_info)
+
+
 @device_guard
 def seg_adain_batch(content_feat: torch.Tensor, style_feat: torch.Tensor, c_labels: torch.Tensor,
                     s_labels: torch.Tensor, prev: Optional[torch.Tensor] = None, return_info: bool = False, *,
-                    content_map: Optional[torch.Tensor] = None, style_map: Optional[torch.Tensor] = None):
+                    content_map: Optional[torch.Tensor] = None, style_map: Optional[torch.Tensor] = None,
+                    differentiable: bool = False):
     """Batched segment AdaIN.  content [N,C,Hc,Wc], style [N,C,Hs,Ws], labels uint8 [N,Hc,Wc] /
     [N,Hs,Ws].  `prev` (same shape as content) is added to the result in the same pass.
     With `return_info` also returns the [N,256,3] int32 table (cnt_c, cnt_s, usable).
     `content_map` / `style_map` (int32 [N*C] plane indices, as in `adain_mapped`) make output plane p read
     `content_feat.flatten(0,1)[content_map[p]]` / `style_feat.flatten(0,1)[style_map[p]]` without
-    materialising the permuted tensors; labels, `prev` and the label table stay those of the output sample."""
+    materialising the permuted tensors; labels, `prev` and the label table stay those of the output sample.
+    Gradients are opt-in: by default a content, style or `prev` that requires grad raises NotImplementedError;
+    with `differentiable=True` the call is recorded for autograd (rpst_seg_adain_bwd computes the content and
+    style gradients, `prev` receives the upstream gradient)."""
     assert content_feat.dim() == 4 and style_feat.dim() == 4
     assert content_feat.shape[:2] == style_feat.shape[:2], "batch/channel mismatch"
+    if differentiable and _needs_grad(content_feat, style_feat, prev):
+        return _seg_adain_grad(content_feat, style_feat, c_labels, s_labels, prev, content_map, style_map, return_info)
     _refuse_grad(content_feat, style_feat, prev)
     out = torch.empty(content_feat.shape, dtype=torch.float32, device=content_feat.device)
     ch, hw = content_feat.shape[1], content_feat.shape[2] * content_feat.shape[3]
@@ -100,14 +165,18 @@ def seg_adain_batch(content_feat: torch.Tensor, style_feat: torch.Tensor, c_labe
 @device_guard
 def seg_adain_concat(prev: torch.Tensor, content_feat: torch.Tensor, style_feat: torch.Tensor, c_labels: torch.Tensor,
                      s_labels: torch.Tensor, *, content_map: Optional[torch.Tensor] = None,
-                     style_map: Optional[torch.Tensor] = None) -> torch.Tensor:
+                     style_map: Optional[torch.Tensor] = None, differentiable: bool = False) -> torch.Tensor:
     """`torch.cat([prev, seg_adain_batch(content_feat, style_feat, c_labels, s_labels)], dim=1)` with the
     segment half written straight into the channel slice of the result (the masked branch of
-    network/adain_rp.py:793, mirroring `adain_concat`).  Maps as in `seg_adain_batch`.  Segment AdaIN has no
-    backward pass; a `prev` that requires grad keeps its gradient through an ordinary `torch.cat`."""
+    network/adain_rp.py:793, mirroring `adain_concat`).  Maps as in `seg_adain_batch`.  A `prev` that requires
+    grad keeps its gradient through an ordinary `torch.cat`; content and style gradients need
+    `differentiable=True` (as in `seg_adain_batch`), which also goes through `torch.cat`."""
     assert content_feat.dim() == 4 and style_feat.dim() == 4
     assert content_feat.shape[:2] == style_feat.shape[:2], "batch/channel mismatch"
     assert prev.dim() == 4 and prev.shape[0] == content_feat.shape[0] and prev.shape[2:] == content_feat.shape[2:]
+    if differentiable and _needs_grad(content_feat, style_feat):
+        return torch.cat([prev, seg_adain_batch(content_feat, style_feat, c_labels, s_labels, content_map=content_map,
+                                                style_map=style_map, differentiable=True)], dim=1)
     _refuse_grad(content_feat, style_feat)
     if torch.is_grad_enabled() and prev.requires_grad:
         return torch.cat([prev, seg_adain_batch(content_feat, style_feat, c_labels, s_labels, content_map=content_map,
@@ -123,26 +192,29 @@ def seg_adain_concat(prev: torch.Tensor, content_feat: torch.Tensor, style_feat:
 
 @device_guard
 def adaptive_instance_normalization_with_segment(content_feat: torch.Tensor, style_feat: torch.Tensor,
-                                                 content_seg_path: LabelArg, style_seg_path: LabelArg) -> torch.Tensor:
+                                                 content_seg_path: LabelArg, style_seg_path: LabelArg, *,
+                                                 differentiable: bool = False) -> torch.Tensor:
     """Drop-in for network/base.py:494 — (1,c,hc,wc), (1,c,hs,ws), two label maps (paths, arrays or
-    tensors) -> (1,c,hc,wc)."""
+    tensors) -> (1,c,hc,wc).  `differentiable` as in `seg_adain_batch`."""
     assert content_feat.shape[0] == 1 and style_feat.shape[0] == 1
     hc, wc = content_feat.shape[2:]
     hs, ws = style_feat.shape[2:]
     cl = load_label_map(content_seg_path, wc, hc, content_feat.device)
     sl = load_label_map(style_seg_path, ws, hs, style_feat.device)
-    return seg_adain_batch(content_feat, style_feat, cl[None], sl[None])
+    return seg_adain_batch(content_feat, style_feat, cl[None], sl[None], differentiable=differentiable)
 
 
 @device_guard
 def do_mask_stylized(content_feat: torch.Tensor, style_feat: torch.Tensor, c_masks: Sequence[LabelArg],
                      s_masks: Sequence[LabelArg], prev: Optional[torch.Tensor] = None, *,
-                     content_map: Optional[torch.Tensor] = None, style_map: Optional[torch.Tensor] = None) -> torch.Tensor:
+                     content_map: Optional[torch.Tensor] = None, style_map: Optional[torch.Tensor] = None,
+                     differentiable: bool = False) -> torch.Tensor:
     """Replacement for the per-sample Python loop network/adain_rp.py:313-319: one launch for the
     whole batch.  `c_masks[i]` / `s_masks[i]` are per-sample label maps (paths/arrays/tensors), or a
-    ready [N,H,W] uint8 tensor.  Plane maps as in `seg_adain_batch`."""
+    ready [N,H,W] uint8 tensor.  Plane maps and `differentiable` as in `seg_adain_batch`."""
     hc, wc = content_feat.shape[2:]
     hs, ws = style_feat.shape[2:]
     dev = content_feat.device
     return seg_adain_batch(content_feat, style_feat, stack_label_maps(c_masks, wc, hc, dev),
-                           stack_label_maps(s_masks, ws, hs, dev), prev, content_map=content_map, style_map=style_map)
+                           stack_label_maps(s_masks, ws, hs, dev), prev, content_map=content_map, style_map=style_map,
+                           differentiable=differentiable)
